@@ -3,6 +3,8 @@
 
   python bench.py --gpus N --steps K --warmup W            this engine (one process per GPU under torchrun)
   python bench.py --impl reference --gpus N --steps K ...  the reference's own CPU implementation (oracle/_ref)
+  python bench.py ... --dump-outputs DIR                    also writes the headline's last timed step as DIR/<name>.npy
+                                                            (inputs are seeded: two builds can be compared output for output)
 
 A "step" = one pass of the hot path over one batch: network forward (conv stack) + device decode +
 class-wise NMS for all images of the batch.  Headline workload = configs[2] of BASELINE.json: YOLOv3 416x416,
@@ -384,6 +386,23 @@ def dropin_latency(dn, sampler, iters=30):
             "do_nms_sort_ms": med["nms"], "candidates": int(num.value), "iters": iters, "clocks": sampler.summary(t_begin, t_end) if sampler else None}
 
 
+def dump_outputs(out_dir, rec, counts):
+    """the last timed step's result as .npy files, so that two builds can be compared output for output: the kept
+    (box, class) records of every image, ordered by (image, box id, class) because the device may emit them in any order,
+    and the per-image candidate counts before NMS.  Integer fields are stored as float64, which holds them exactly.
+    Under torchrun, rank 0 writes the gathered records of every rank (global image numbers) but only its own images'
+    counts: counts.npy covers images 0..BATCH-1."""
+    os.makedirs(out_dir, exist_ok=True)
+    rec = rec[np.lexsort((rec["cls"], rec["box_id"], rec["image"]))]
+    arrays = {"counts": np.asarray(counts, np.float64), "image": rec["image"].astype(np.float64),
+              "box_id": rec["box_id"].astype(np.float64), "cls": rec["cls"].astype(np.float64),
+              "prob": rec["prob"].astype(np.float32), "objectness": rec["objectness"].astype(np.float32),
+              "bbox": np.stack([rec["bbox"][k] for k in "xywh"], axis=1).astype(np.float32)}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 _T0 = time.time()
 
 
@@ -436,6 +455,8 @@ def main_engine(args):
     launches = dn.lib.b200_launch_count() - launches0
     cand = float(np.mean(list(run.counts)))
     value = world * BATCH * args.steps / (ms / 1000.0)
+    if args.dump_outputs and rank == 0:               # before drain(): it overwrites the records and counts of the last step
+        dump_outputs(args.dump_outputs, np.ctypeslib.as_array(run.out, shape=(run.max_out,))[:nrec], list(run.counts))
     run.drain()                                       # the forward pass pre-enqueued for a step that will not come
     total_records = int(nrec)                         # on rank 0 with the gather on: the records of ALL ranks for the last step
 
@@ -593,12 +614,19 @@ if __name__ == "__main__":
         faulthandler.dump_traceback_later(int(os.environ["B200_BENCH_WATCHDOG"]), exit=True)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline and of the two e2e loops, exactly; the bounded sections clamp it and report the "
+                         "count they ran: c4 to 3..10, other_configs to 5..10, --impl reference to 1..8 (cpu_baseline always times 4)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip C4, the other configurations and the drop-in latency")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records and counts of the headline's last timed step to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs covers this engine's records only, not those of --impl reference")
     if a.impl == "reference":
         main_reference(a)
     else:
