@@ -33,8 +33,8 @@ def conv(f, k, s, bn=1, act="leaky"):
     return t + f"filters={f}\nsize={k}\nstride={s}\npad=1\nactivation={act}\n"
 
 
-def from_table(path, head_filters, head_block, yolo_masks=None):
-    rows = open(path).read().splitlines()[1:]
+def from_table(path, head_filters, head_block, yolo_masks=None, rows=None):
+    rows = open(path).read().splitlines()[1:][:rows]
     out, nyolo = [], 0
     for i, row in enumerate(rows):
         tok = row.split()
@@ -113,7 +113,26 @@ def yolov3_tiny(w=416, h=416, batch=1):
     return net_section(w, h, batch) + "\n" + "\n".join(L)
 
 
-MODELS = {"yolov3": yolov3, "yolov2": yolov2, "yolov1": yolov1, "yolov3-tiny": yolov3_tiny}
+# ImageNet classifiers: the detectors' own backbones with darknet's classification tail (1000-way linear 1x1 conv, global
+# average pool, softmax, and the [cost] layer training needs and inference skips).  Darknet-53 pools before the 1x1,
+# Darknet-19 after it.
+CLASSIFIER_TAIL = "[softmax]\ngroups=1\n", "[cost]\ntype=sse\n"
+
+
+def darknet53(w=256, h=256, batch=1):
+    body = from_table(os.path.join(TABLES, "yolov3.txt"), set(), None, rows=75)
+    tail = ["[avgpool]\n", conv(1000, 1, 1, bn=0, act="linear"), *CLASSIFIER_TAIL]
+    return net_section(w, h, batch) + "\n" + "\n".join(body + tail)
+
+
+def darknet19(w=224, h=224, batch=1):
+    body = from_table(os.path.join(TABLES, "yolov2.txt"), set(), None, rows=23)
+    tail = [conv(1000, 1, 1, bn=0, act="linear"), "[avgpool]\n", *CLASSIFIER_TAIL]
+    return net_section(w, h, batch) + "\n" + "\n".join(body + tail)
+
+
+MODELS = {"yolov3": yolov3, "yolov2": yolov2, "yolov1": yolov1, "yolov3-tiny": yolov3_tiny, "darknet19": darknet19,
+          "darknet53": darknet53}
 
 if __name__ == "__main__":
     for name, fn in MODELS.items():

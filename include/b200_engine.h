@@ -184,6 +184,18 @@ void b200_submit_batch(network *net, const float *input);
 int  b200_detect_submitted(network *net, const float *next_input, int w, int h, float thresh, float nms_thresh, int relative,
                            b200_det *out, int max_out, int *counts);
 
+/* ---- classifiers (Darknet-19, Darknet-53: networks ending in [softmax]) ------------------------------------------------ */
+/* network_predict + top_k for EVERY image on the device; the network must end in [softmax] (groups = 1), 1 <= top <= 64.
+ * classes[b*top + j], probs[b*top + j]: the j-th entry of top_k over image b's probabilities.  input: host fp32 NCHW, or
+ * B200_INPUT_RESIDENT (the device input buffer, e.g. after b200_letterbox_batch_u8).  Returns the number of images, -1 on a
+ * network that does not end in [softmax] or a `top` out of range.  (b200_detect_batch / b200_detect_submitted return -1 on
+ * such a network.) */
+int  b200_classify_batch(network *net, const float *input, int top, int *classes, float *probs);
+/* the double-buffered loop of b200_detect_submitted, same contract, for classifiers (after b200_submit_batch) */
+int  b200_classify_submitted(network *net, const float *next_input, int top, int *classes, float *probs);
+/* the device top-k on caller rows (rows x n, host), exposed for parity tests like b200_nms_sort_arrays */
+void b200_top_k_arrays(const float *probs, int rows, int n, int top, int *classes);
+
 /* ---- multi-GPU: image-sharded replicas, one process per GPU (SURVEY.md §8e) --------------------------------------------
  * Every process parses the same cfg; rank `root` alone loads the .weights file.  NCCL is resolved at run time (dlopen of
  * libnccl.so.2).  The 128-byte id made by b200_comm_unique_id on one rank reaches the others by any out-of-band channel

@@ -187,6 +187,7 @@ int    find_arg(int argc, char *argv[], char *arg);                         /* r
 int    find_int_arg(int argc, char **argv, char *arg, int def);             /* ref :766  utils.c:133       */
 float  find_float_arg(int argc, char **argv, char *arg, float def);         /* ref :767  utils.c:148       */
 char  *find_char_arg(int argc, char **argv, char *arg, char *def);          /* ref :769  utils.c:163       */
+void   top_k(float *a, int n, int k, int *index);                          /* utils.c top_k               */
 char  *basecfg(char *cfgfile);                                              /* ref :770  utils.c:179       */
 char  *fgetl(FILE *fp);                                                     /* ref :773  utils.c:335       */
 void   strip(char *s);                                                      /* ref :774  utils.c:302       */

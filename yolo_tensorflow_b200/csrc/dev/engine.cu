@@ -98,7 +98,7 @@ static bool layer_launches(const b200_engine *e, const network *net, int j)
     case UPSAMPLE: return !d.up_away;
     case MAXPOOL: return !d.pool_away;
     case ROUTE: return d.kernel == "route_copy";
-    case DROPOUT: return false;
+    case DROPOUT: case COST: return false;
     default: return true;
     }
 }
@@ -112,7 +112,7 @@ static void writers_of(const b200_engine *e, const network *net, int j, std::vec
     case SHORTCUT: if (d.fused_away) { out.push_back(j - 1); return; } break;
     case UPSAMPLE: if (d.up_away) { out.push_back(j - 1); return; } break;
     case MAXPOOL: if (d.pool_away) { out.push_back(j - 1); return; } break;
-    case DROPOUT: if (j > 0) { writers_of(e, net, j - 1, out); return; } break;
+    case DROPOUT: case COST: if (j > 0) { writers_of(e, net, j - 1, out); return; } break;
     case ROUTE:
         for (int k = 0; k < l.n; ++k) writers_of(e, net, l.input_layers[k], out);
         if (d.kernel == "route_copy") out.push_back(j);
@@ -219,6 +219,18 @@ static void build_engine_device_state(b200_engine *e, network *net)
         return TView{(unsigned char *)rd.out.p + (size_t)place_off[sidx] * dt_size(dtype), e->cap, sl.out_h, sl.out_w, sl.out_c, rl.out_c, dtype};
     };
 
+    // ---- classifier tail: the [softmax] the network ends in, and the convolution feeding it (directly or through [avgpool]) ----
+    auto only_consumer_is = [&](int j, LAYER_TYPE t) { return j + 1 < net->n && cons[j].size() == 1 && cons[j][0] == j + 1 && net->layers[j + 1].type == t; };
+    e->cls_layer = -1;
+    {
+        int last = net->n - 1;
+        while (last > 0 && net->layers[last].type == COST) --last;
+        if (net->layers[last].type == SOFTMAX) e->cls_layer = last;
+    }
+    for (int i = 0; i < net->n; ++i)
+        e->L[i].cls_logits = net->layers[i].type == CONVOLUTIONAL &&
+                             (only_consumer_is(i, SOFTMAX) || (only_consumer_is(i, AVGPOOL) && only_consumer_is(i + 1, SOFTMAX)));
+
     // ---- output views ------------------------------------------------------------------------------
     for (int i = 0; i < net->n; ++i) {
         const layer &l = net->layers[i];
@@ -230,10 +242,13 @@ static void build_engine_device_state(b200_engine *e, network *net)
         if (l.type == CONVOLUTIONAL && e->precision == B200_PREC_BF16 && i + 1 < net->n && cons[i].size() == 1 &&
             (net->layers[i + 1].type == YOLO || net->layers[i + 1].type == REGION))
             dtype = DT_F32;                        // head logits stay fp32: no quantisation before the decode
+        if (d.cls_logits || (l.type == AVGPOOL && only_consumer_is(i, SOFTMAX)))
+            dtype = DT_F32;                        // so do a classifier's logits, up to its [softmax]
         switch (l.type) {
         case CONVOLUTIONAL: {
-            // row pitch padded to 16 filters (255 -> 256): keeps every pixel row 16-byte aligned for vector stores
-            int ld = (int)align_up(l.out_c, 16);
+            // row pitch padded to 16 filters (255 -> 256): keeps every pixel row 16-byte aligned for vector stores; a classifier's
+            // logits to 64 (1000 -> 1024), whole 64-filter tiles of the tcgen05 GEMM like the connected layer's
+            int ld = (int)align_up(l.out_c, d.cls_logits ? 64 : 16);
             if (d.fused_into >= 0) {            // written straight into the shortcut's buffer, never materialised
                 d.out = TView{nullptr, e->cap, l.out_h, l.out_w, l.out_c, ld, dtype};
                 d.owns_out = false;
@@ -259,10 +274,22 @@ static void build_engine_device_state(b200_engine *e, network *net)
                 d.owns_out = true;
             }
             break;
-        case DROPOUT:
+        case DROPOUT: case COST:                   // identities at inference (cost: network_predict clears net->truth)
             d.out = e->L[i - 1].out; d.owns_out = false;
             d.head_out = e->L[i - 1].head_out;
             break;
+        case AVGPOOL:
+            d.out = TView{dev_alloc((size_t)e->cap * l.out_c * dt_size(dtype)), e->cap, 1, 1, l.out_c, l.out_c, dtype};
+            d.owns_out = true;
+            break;
+        case SOFTMAX:
+            if (i == 0 || net->layers[i - 1].out_h != 1 || net->layers[i - 1].out_w != 1 || net->layers[i - 1].out_c != l.inputs) {
+                fprintf(stderr, "b200-darknet: [softmax] (layer %d) needs a 1 x 1 map as its input, e.g. after [avgpool]; "
+                                "layer %d outputs %d x %d x %d\n", i, i - 1, i ? net->layers[i - 1].out_w : 0,
+                        i ? net->layers[i - 1].out_h : 0, i ? net->layers[i - 1].out_c : 0);
+                abort();
+            }
+            // fall through: an fp32 [batch][outputs] head like the detection layers'
         case CONNECTED: case YOLO: case REGION: case DETECTION:
             d.head_out = (float *)dev_alloc(floats * sizeof(float));
             d.out = TView{d.head_out, e->cap, 1, 1, l.outputs, l.outputs, DT_F32};
@@ -290,7 +317,7 @@ static void build_engine_device_state(b200_engine *e, network *net)
         const layer &l = net->layers[i];
         DevLayer &d = e->L[i];
         if (l.type == CONVOLUTIONAL) {
-            d.cout_pad = (int)align_up(l.n, 16);
+            d.cout_pad = (int)align_up(l.n, d.cls_logits ? 64 : 16);
             d.w_bytes = (size_t)d.cout_pad * l.size * l.size * l.c * esize;
             d.w_off = off; off = align_up(off + d.w_bytes, 256);
             d.scale_off = off; off = align_up(off + d.cout_pad * sizeof(float), 256);
@@ -423,6 +450,9 @@ static void build_engine_device_state(b200_engine *e, network *net)
             break;
         }
         case YOLO: d.kernel = "yolo_forward"; break;
+        case AVGPOOL: d.kernel = "avgpool"; break;
+        case SOFTMAX: d.kernel = "softmax"; break;
+        case COST: d.kernel = "alias"; break;
         case REGION: d.kernel = "region_forward"; break;
         case DETECTION: d.kernel = "detection_forward"; break;
         default: break;
@@ -560,7 +590,7 @@ extern "C" b200_engine *b200_engine_create(network *net, int precision)
     e->conv_backend = 0;
     e->head_sync = 1;
     e->L.resize(net->n);
-    for (auto &d : e->L) { d = DevLayer(); d.tc = nullptr; d.head_out = nullptr; d.w = nullptr; d.stem = false; d.owns_out = false; d.fused_into = -1; d.fused_away = false; d.block_head = false; d.up_fused = false; d.up_away = false; d.fc_tmp = nullptr; d.pool_fused = false; d.pool_away = false; d.reorg_table = nullptr; }
+    for (auto &d : e->L) { d = DevLayer(); d.tc = nullptr; d.head_out = nullptr; d.w = nullptr; d.stem = false; d.owns_out = false; d.fused_into = -1; d.fused_away = false; d.block_head = false; d.up_fused = false; d.up_away = false; d.fc_tmp = nullptr; d.pool_fused = false; d.pool_away = false; d.reorg_table = nullptr; d.cls_logits = false; }
     e->fusion = b200_get_default_fusion();
     e->stream = nullptr; e->d_input = nullptr; e->d_input_next = nullptr; e->submitted = 0; e->arena = nullptr; e->xfer = nullptr; e->d_heads = nullptr;
     e->in_view = TView{nullptr, 0, 0, 0, 0, 0, 0};
@@ -570,6 +600,7 @@ extern "C" b200_engine *b200_engine_create(network *net, int precision)
     e->d_raw = nullptr; e->raw_cap = 0; e->d_lb_items = nullptr; e->d_im_dims[0] = e->d_im_dims[1] = nullptr; e->dims_cur = 0; e->dims_pending = 0;
     e->h_box = e->h_obj = e->h_prob = nullptr; e->h_id = nullptr; e->h_cap = 0;
     e->boxes_per_image = 0; e->classes = 0; e->has_tree = false; e->d_map = nullptr;
+    e->cls_layer = -1; e->d_top_cls = nullptr; e->d_top_prob = nullptr;
     // Parsing a cfg (layer table, shapes) works on a machine without a GPU; anything that computes does not.
     if (cuda_usable()) build_engine_device_state(e, net);
     else e->device = -1;
@@ -607,7 +638,7 @@ extern "C" void b200_engine_destroy(b200_engine *e)
             if (d.tc) conv_tc_plan_destroy(d.tc);
             if (d.owns_out) cudaFree(d.out.p);
             cudaFree(d.fc_tmp); cudaFree(d.reorg_table);
-            if (d.head_out && d.type != DROPOUT) cudaFree(d.head_out);
+            if (d.head_out && d.type != DROPOUT && d.type != COST) cudaFree(d.head_out);
         }
         cudaFree(e->d_input); cudaFree(e->d_input_next); cudaEventDestroy(e->submit_done); cudaFree(e->in_view.p); cudaFree(e->arena); cudaFree(e->xfer); cudaFree(e->d_heads);
         cudaFree(e->cand.box); cudaFree(e->cand.obj); cudaFree(e->cand.prob); cudaFree(e->cand.id); cudaFree(e->cand.count);
@@ -615,6 +646,7 @@ extern "C" void b200_engine_destroy(b200_engine *e)
         cudaFree(e->nms_scratch.mask); cudaFree(e->d_records); cudaFree(e->d_record_count);
         for (int *p : e->tree_arrays) cudaFree(p);
         cudaFree(e->d_map);
+        cudaFree(e->d_top_cls); cudaFree(e->d_top_prob);
         cudaFree(e->d_raw); cudaFree(e->d_lb_items); cudaFree(e->d_im_dims[0]); cudaFree(e->d_im_dims[1]);
         cudaFreeHost(e->h_box); cudaFreeHost(e->h_obj); cudaFreeHost(e->h_prob); cudaFreeHost(e->h_id);
         for (auto &ev : e->copy_done) cudaEventDestroy(ev);
@@ -774,7 +806,9 @@ static void run_layer(b200_engine *e, network *net, int i, int batch)
             }
         }
         break;
-    case DROPOUT: break;
+    case DROPOUT: case COST: break;
+    case AVGPOOL: launch_avgpool(in, out, s); break;
+    case SOFTMAX: launch_softmax(in, d.head_out, batch, l.groups, l.temperature, s); break;
     case LOCAL:
         if (d.tc && e->conv_backend == 0) launch_conv_tc(d.tc, s);
         else launch_local(in, out, d.w, d.lbias, l.size, l.stride, l.pad, act_id(l.activation), s);
@@ -1347,11 +1381,20 @@ static int detect_core(b200_engine *e, network *net, int first, int w, int h, fl
     return n;
 }
 
+// a classifier (a network ending in [softmax]) has no detection head: the batched detection entry points refuse it
+static bool refuse_classifier(const b200_engine *e, const char *what)
+{
+    if (e->cls_layer < 0) return false;
+    fprintf(stderr, "b200-darknet: %s: the network ends in [softmax] and has no detection head; use b200_classify_batch\n", what);
+    return true;
+}
+
 extern "C" int b200_detect_batch(network *net, const float *input, int w, int h, float thresh, float nms_thresh,
                                  int relative, b200_det *out, int max_out, int *counts)
 {
     b200_engine *e = b200_engine_of(net);
     need_device(e, "b200_detect_batch");
+    if (refuse_classifier(e, "b200_detect_batch")) return -1;
     const int first = input ? stage_input(e, net, input) : 0;
     return detect_core(e, net, first, w, h, thresh, nms_thresh, relative, out, max_out, counts);
 }
@@ -1464,11 +1507,26 @@ extern "C" void b200_submit_batch(network *net, const float *input)
     e->submitted = 1;
 }
 
+// the serving loops' step after the current batch's tail is enqueued: submit `next_input` (may be NULL) and enqueue its forward pass
+static void enqueue_next_batch(b200_engine *e, network *net, const float *next_input)
+{
+    if (!next_input) return;
+    b200_submit_batch(net, next_input);
+    if (next_input == B200_INPUT_RESIDENT) return;                                   // forward enqueued by the submit
+    float *t = e->d_input; e->d_input = e->d_input_next; e->d_input_next = t;
+    B200_CHECK(cudaStreamWaitEvent(e->stream, e->submit_done, 0));
+    const int use_raw = (!e->head_sync && e->raw_decode_ok && !e->heads.empty()) ? 1 : 0;
+    adopt_letterbox_dims(e);
+    forward_layers(e, net, 0, net->n, use_raw != 0);
+    e->fwd_enqueued = 1;
+}
+
 extern "C" int b200_detect_submitted(network *net, const float *next_input, int w, int h, float thresh, float nms_thresh,
                                      int relative, b200_det *out, int max_out, int *counts)
 {
     b200_engine *e = b200_engine_of(net);
     need_device(e, "b200_detect_submitted");
+    if (refuse_classifier(e, "b200_detect_submitted")) return -1;
     if (!e->submitted) { fprintf(stderr, "b200-darknet: b200_detect_submitted without a submitted batch\n"); abort(); }
     int first = net->n;                                                              // forward already enqueued by the previous call?
     if (!e->fwd_enqueued) {
@@ -1480,17 +1538,79 @@ extern "C" int b200_detect_submitted(network *net, const float *next_input, int 
     // Once this batch's decode / NMS / collect are in the stream, the NEXT batch's copy is submitted and its whole forward pass
     // is enqueued behind them; the results of this batch are then read back on a separate stream while that forward runs.
     // (Waiting for the results first left the GPU idle for the two D2H round trips: ~0.25 ms of every 5 ms step.)
-    return detect_core(e, net, first, w, h, thresh, nms_thresh, relative, out, max_out, counts, [&] {
-        if (!next_input) return;
-        b200_submit_batch(net, next_input);
-        if (next_input == B200_INPUT_RESIDENT) return;                                   // forward enqueued by the submit
+    return detect_core(e, net, first, w, h, thresh, nms_thresh, relative, out, max_out, counts, [&] { enqueue_next_batch(e, net, next_input); });
+}
+
+// ----------------------------------------------------------------------------------------------------
+// classifiers: network_predict + top_k (predict_classifier, examples/classifier.c) for every image of the batch, the ranking
+// on the device; only `top` (class, probability) pairs per image cross PCIe.
+// ----------------------------------------------------------------------------------------------------
+static bool classify_args_ok(const b200_engine *e, const network *net, int top, const char *what)
+{
+    if (e->cls_layer < 0) {
+        fprintf(stderr, "b200-darknet: %s: the network does not end in [softmax]\n", what);
+        return false;
+    }
+    const layer &l = net->layers[e->cls_layer];
+    if (l.groups != 1) {
+        fprintf(stderr, "b200-darknet: %s: the final [softmax] has groups = %d; ranking needs groups = 1\n", what, l.groups);
+        return false;
+    }
+    if (top < 1 || top > 64 || top > l.outputs) {
+        fprintf(stderr, "b200-darknet: %s: top = %d is outside 1..%d\n", what, top, l.outputs < 64 ? l.outputs : 64);
+        return false;
+    }
+    return true;
+}
+
+// forward from layer `first` (net->n: already in the stream) + top-k on the compute stream; `after_tail` enqueues the next
+// batch behind them before the results are read back on their own stream (the pattern of detect_core)
+template <typename F>
+static int classify_core(b200_engine *e, network *net, int first, int top, int *classes, float *probs, F after_tail)
+{
+    const int batch = logical_batch(e, net);
+    const layer &l = net->layers[e->cls_layer];
+    if (!e->d_top_cls) {
+        e->d_top_cls = (int *)dev_alloc((size_t)e->cap * 64 * sizeof(int));
+        e->d_top_prob = (float *)dev_alloc((size_t)e->cap * 64 * sizeof(float));
+    }
+    if (first < net->n) adopt_letterbox_dims(e);
+    forward_layers(e, net, first, net->n);
+    launch_topk(e->L[e->cls_layer].head_out, batch, l.outputs, l.outputs, top, e->d_top_cls, e->d_top_prob, e->stream);
+    B200_CHECK(cudaEventRecord(e->tail_done, e->stream));
+    B200_CHECK(cudaStreamWaitEvent(e->d2h_stream, e->tail_done, 0));
+    after_tail();
+    B200_CHECK(cudaMemcpyAsync(classes, e->d_top_cls, (size_t)batch * top * sizeof(int), cudaMemcpyDeviceToHost, e->d2h_stream));
+    B200_CHECK(cudaMemcpyAsync(probs, e->d_top_prob, (size_t)batch * top * sizeof(float), cudaMemcpyDeviceToHost, e->d2h_stream));
+    B200_CHECK(cudaStreamSynchronize(e->d2h_stream));
+    return batch;
+}
+
+extern "C" int b200_classify_batch(network *net, const float *input, int top, int *classes, float *probs)
+{
+    b200_engine *e = b200_engine_of(net);
+    need_device(e, "b200_classify_batch");
+    if (!classify_args_ok(e, net, top, "b200_classify_batch")) return -1;
+    const int first = (input && input != B200_INPUT_RESIDENT) ? stage_input(e, net, input) : 0;
+    const int n = classify_core(e, net, first, top, classes, probs, [] {});
+    B200_CHECK(cudaStreamSynchronize(e->stream));
+    return n;
+}
+
+extern "C" int b200_classify_submitted(network *net, const float *next_input, int top, int *classes, float *probs)
+{
+    b200_engine *e = b200_engine_of(net);
+    need_device(e, "b200_classify_submitted");
+    if (!classify_args_ok(e, net, top, "b200_classify_submitted")) return -1;
+    if (!e->submitted) { fprintf(stderr, "b200-darknet: b200_classify_submitted without a submitted batch\n"); abort(); }
+    int first = net->n;
+    if (!e->fwd_enqueued) {
         float *t = e->d_input; e->d_input = e->d_input_next; e->d_input_next = t;
         B200_CHECK(cudaStreamWaitEvent(e->stream, e->submit_done, 0));
-        const int use_raw = (!e->head_sync && e->raw_decode_ok && !e->heads.empty()) ? 1 : 0;
-        adopt_letterbox_dims(e);
-        forward_layers(e, net, 0, net->n, use_raw != 0);
-        e->fwd_enqueued = 1;
-    });
+        first = 0;
+    }
+    e->submitted = 0; e->fwd_enqueued = 0;
+    return classify_core(e, net, first, top, classes, probs, [&] { enqueue_next_batch(e, net, next_input); });
 }
 
 // device NMS on caller-provided host arrays (the kernel behind do_nms_sort / do_nms_obj).  Stream, scratch slab and staging
@@ -1542,4 +1662,17 @@ extern "C" void b200_nms_obj_arrays(const float *boxes, float *objectness, int n
     B200_CHECK(cudaMemcpyAsync(objectness, p.d_val, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, p.stream));
     B200_CHECK(cudaStreamSynchronize(p.stream));
     if (suppressed) for (int i = 0; i < n; ++i) suppressed[i] = (before[i] != 0.f && objectness[i] == 0.f) ? 1 : 0;
+}
+
+extern "C" void b200_top_k_arrays(const float *probs, int rows, int n, int top, int *classes)
+{
+    if (rows <= 0 || n <= 0 || top < 1 || top > 64 || top > n) {
+        fprintf(stderr, "b200-darknet: b200_top_k_arrays: needs rows >= 1 and 1 <= top <= min(n, 64)\n");
+        abort();
+    }
+    NmsHostPath &p = nms_prepare(0, (size_t)rows * n, (size_t)rows * top);
+    B200_CHECK(cudaMemcpyAsync(p.d_val, probs, (size_t)rows * n * sizeof(float), cudaMemcpyHostToDevice, p.stream));
+    launch_topk(p.d_val, rows, n, n, top, p.d_cls, nullptr, p.stream);
+    B200_CHECK(cudaMemcpyAsync(classes, p.d_cls, (size_t)rows * top * sizeof(int), cudaMemcpyDeviceToHost, p.stream));
+    B200_CHECK(cudaStreamSynchronize(p.stream));
 }

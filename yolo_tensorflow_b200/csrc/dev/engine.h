@@ -29,6 +29,7 @@ struct DevLayer {
     bool pool_away;            // [maxpool] performed inside the stem kernel
     bool block_head;           // 1x1 conv computed inside the following 3x3's kernel (fused residual block): launches nothing
     int *reorg_table;          // [reorg]: the per-image permutation as (source, destination) offset pairs on the device
+    bool cls_logits;           // conv feeding a classifier's [softmax] (directly or through [avgpool]): fp32, rows padded to 64 filters
     std::string kernel;
 };
 
@@ -78,6 +79,9 @@ struct b200_engine {
     unsigned char *d_raw; size_t raw_cap;            // b200_letterbox_batch*: source images on the device
     LetterboxItem *d_lb_items; int *d_im_dims[2];    // per-image resize geometry / original sizes (box correction):
     int dims_cur, dims_pending;                      // [dims_cur] belongs to the batch whose forward pass was enqueued last, the other slot to the next letterbox call
+    // classifiers: the [softmax] the network ends in (or -1) and the device top-k results of b200_classify_*
+    int cls_layer;
+    int *d_top_cls; float *d_top_prob;
     // host staging for one image's candidates
     float *h_box, *h_obj, *h_prob; int *h_id; int h_cap;
 };

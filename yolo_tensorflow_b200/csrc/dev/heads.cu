@@ -7,6 +7,7 @@
 // of the region layer (region_layer.c:182-185 -> blas.c:305-332).  The NHWC->NCHW transpose is fused into
 // the same pass, so logits are read once and activations written once: 2 x outputs x 4 bytes of HBM traffic.
 #include "kernels.h"
+#include "softmax.cuh"
 #include <cfloat>
 
 static const int kThreads = 256;
@@ -158,17 +159,8 @@ __global__ void region_forward_kernel(const T *__restrict__ in, float *__restric
         }
         for (int g = 0; g < groups; ++g) {
             const int off = coords + 1 + (gsize ? goff[g] : 0), sz = gsize ? gsize[g] : classes;
-            float largest = -FLT_MAX;
-            for (int j = lane; j < sz; j += 32) largest = fmaxf(largest, Elem<T>::load(src + off + j));
-            for (int o = 16; o; o >>= 1) largest = fmaxf(largest, __shfl_xor_sync(0xffffffffu, largest, o));
-            float sum = 0.f;
-            for (int j = lane; j < sz; j += 32) {
-                const float e = (float)exp((double)(Elem<T>::load(src + off + j) - largest));
-                sum += e;
-                dst[(size_t)(off + j) * HW] = e;
-            }
-            for (int o = 16; o; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
-            for (int j = lane; j < sz; j += 32) dst[(size_t)(off + j) * HW] /= sum;
+            group_softmax(sz, 1.f, lane, 32, [&](int j) { return Elem<T>::load(src + off + j); },
+                          [&](int j) -> float & { return dst[(size_t)(off + j) * HW]; }, warp_all_max, warp_all_sum);
         }
     }
 }
@@ -202,17 +194,8 @@ region_forward_tiled_kernel(const T *__restrict__ in, float *__restrict__ out, i
             }
             for (int g = 0; g < groups; ++g) {
                 const int off = coords + 1 + (gsize ? goff[g] : 0), sz = gsize ? gsize[g] : classes;
-                float largest = -FLT_MAX;
-                for (int j = lane; j < sz; j += 32) largest = fmaxf(largest, Elem<T>::load(src + off + j));
-                for (int o = 16; o; o >>= 1) largest = fmaxf(largest, __shfl_xor_sync(0xffffffffu, largest, o));
-                float sum = 0.f;
-                for (int j = lane; j < sz; j += 32) {
-                    const float e = (float)exp((double)(Elem<T>::load(src + off + j) - largest));
-                    sum += e;
-                    tile[(off + j) * 33 + b] = e;
-                }
-                for (int o = 16; o; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
-                for (int j = lane; j < sz; j += 32) tile[(off + j) * 33 + b] /= sum;
+                group_softmax(sz, 1.f, lane, 32, [&](int j) { return Elem<T>::load(src + off + j); },
+                              [&](int j) -> float & { return tile[(off + j) * 33 + b]; }, warp_all_max, warp_all_sum);
             }
         }
         __syncthreads();

@@ -97,6 +97,14 @@ void launch_detection_forward(const float *in, float *out, int batch, int output
 // l.batch == 2: item 0 <- mean(item 0, horizontally flipped item 1), in place (yolo_layer.c:290-314, region_layer.c:368-390)
 void launch_avg_flipped(float *head_out, int w, int h, int anchors, int entries, int outputs, cudaStream_t s);
 
+// ---- classifier tail (classify.cu) ---------------------------------------------------------------------
+// [avgpool]: in NHWC (any h, w, ld >= c), out (n, 1, 1, c) of either dtype: the mean over the pixels, fp32 sum
+void launch_avgpool(TView in, TView out, cudaStream_t s);
+// [softmax] over `groups` equal slices of in's c channels (in must be a 1 x 1 map); out fp32 [batch][c]
+void launch_softmax(TView in, float *out, int batch, int groups, float temp, cudaStream_t s);
+// top_k of utils.c on each of `rows` rows of n values (row pitch ld): classes[r*k + j] and (if not NULL) probs[r*k + j]
+void launch_topk(const float *a, int rows, int n, int ld, int k, int *classes, float *probs, cudaStream_t s);
+
 // ---- decode + NMS (decode.cu, nms.cu) --------------------------------------------------------------
 struct HeadDesc {            // one per YOLO/REGION/DETECTION layer, device-resident copy lives in the engine
     int type;                // LAYER_TYPE value

@@ -118,6 +118,24 @@ char *basecfg(char *cfgfile)                       /* utils.c:179-191: file name
     return c;
 }
 
+/* utils.c top_k: the k largest entries of a[n], descending, by insertion with a strict `>` (what predict_classifier
+ * and classify() rank with).  An entry displaced from slot j moves on only past strictly smaller entries, so equal values do not
+ * always keep index order (e.g. {5, 5, 3} then 6 gives 6, a[1], a[0]); the device top-k reproduces exactly this order. */
+void top_k(float *a, int n, int k, int *index)
+{
+    for (int j = 0; j < k; ++j) index[j] = -1;
+    for (int i = 0; i < n; ++i) {
+        int curr = i;
+        for (int j = 0; j < k; ++j) {
+            if (index[j] < 0 || a[curr] > a[index[j]]) {
+                int swap = curr;
+                curr = index[j];
+                index[j] = swap;
+            }
+        }
+    }
+}
+
 /* ---- option_list.c ------------------------------------------------------------------------------------------------------ */
 typedef struct { char *key, *val; int used; } kvp;                 /* option_list.h:6-10 */
 

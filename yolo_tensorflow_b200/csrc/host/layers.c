@@ -308,6 +308,70 @@ static layer dropout_layer_(cfg_section *opt, shape_cursor cur)
     return l;
 }
 
+/* [avgpool]: parser.c parse_avgpool + avgpool_layer.c make_avgpool_layer (global average pool of the classifiers) */
+static layer avgpool_layer_(cfg_section *opt, shape_cursor cur)
+{
+    (void)opt;
+    layer l = {0};
+    l.type = AVGPOOL;
+    need_image(cur, "avgpool");
+    l.batch = cur.batch; l.w = cur.w; l.h = cur.h; l.c = cur.c;
+    fprintf(stderr, "avg                     %4d x%4d x%4d   ->  %4d\n", l.w, l.h, l.c, l.c);
+    l.out_w = 1; l.out_h = 1; l.out_c = l.c;
+    l.outputs = l.out_c;
+    l.inputs  = l.h * l.w * l.c;
+    l.output  = host_floats((size_t)l.batch * l.outputs);
+    return l;
+}
+
+/* [softmax]: parser.c parse_softmax + softmax_layer.c make_softmax_layer */
+static layer softmax_layer_(cfg_section *opt, shape_cursor cur)
+{
+    layer l = {0};
+    l.type = SOFTMAX;
+    l.groups = cfg_int_quiet(opt, "groups", 1);
+    if (l.groups < 1 || cur.inputs % l.groups != 0) fatal("softmax groups must divide the layer's inputs");
+    fprintf(stderr, "softmax                                        %4d\n", cur.inputs);
+    l.batch = cur.batch;
+    l.inputs = l.outputs = cur.inputs;
+    l.output = host_floats((size_t)l.batch * l.outputs);
+    l.cost = host_floats(1);
+    l.temperature = cfg_float_quiet(opt, "temperature", 1);
+    if (cfg_str(opt, "tree", 0)) fatal("softmax tree= (WordTree classifiers) is outside the inference path");
+    l.w = cur.w; l.h = cur.h; l.c = cur.c;
+    l.spatial = (int)cfg_float_quiet(opt, "spatial", 0);
+    if (l.spatial) fatal("softmax spatial= is outside the inference path");
+    (void)cfg_int_quiet(opt, "noloss", 0);                  /* training only */
+    return l;
+}
+
+/* [cost]: parser.c parse_cost + cost_layer.c make_cost_layer.  Identity at inference: network_predict clears net->truth, so
+ * forward_cost_layer returns at once; the device engine aliases it to its input. */
+static layer cost_layer_(cfg_section *opt, shape_cursor cur)
+{
+    static const struct { const char *name; COST_TYPE t; } types[] = {
+        {"sse", SSE}, {"masked", MASKED}, {"smooth", SMOOTH}, {"L1", L1}, {"seg", SEG}, {"wgan", WGAN},
+    };
+    layer l = {0};
+    l.type = COST;
+    const char *type = cfg_str(opt, "type", "sse");
+    l.cost_type = SSE;
+    size_t k = 0;
+    while (k < sizeof types / sizeof types[0] && strcmp(type, types[k].name) != 0) ++k;
+    if (k < sizeof types / sizeof types[0]) l.cost_type = types[k].t;
+    else fprintf(stderr, "Couldn't find cost type %s, going with SSE\n", type);          /* cost_layer.c get_cost_type */
+    l.scale = cfg_float_quiet(opt, "scale", 1);
+    fprintf(stderr, "cost                                           %4d\n", cur.inputs);
+    l.batch = cur.batch;
+    l.inputs = l.outputs = cur.inputs;
+    l.output = host_floats((size_t)l.batch * l.outputs);
+    l.cost = host_floats(1);
+    l.ratio = cfg_float_quiet(opt, "ratio", 0);
+    l.noobject_scale = cfg_float_quiet(opt, "noobj", 1);
+    l.thresh = cfg_float_quiet(opt, "thresh", 0);
+    return l;
+}
+
 /* [yolo]: parser.c:303-339 + yolo_layer.c:13-61 */
 static layer yolo_layer_(cfg_section *opt, shape_cursor cur)
 {
@@ -436,6 +500,8 @@ int build_layer(const char *type, cfg_section *opt, shape_cursor cur, layer *out
         {"[shortcut]", 0, shortcut_layer_},          {"[reorg]", 0, reorg_layer_},
         {"[dropout]", 0, dropout_layer_},            {"[yolo]", 0, yolo_layer_},
         {"[region]", 0, region_layer_},              {"[detection]", 0, detection_layer_},
+        {"[avgpool]", "[avg]", avgpool_layer_},      {"[softmax]", "[soft]", softmax_layer_},
+        {"[cost]", 0, cost_layer_},
     };
     for (size_t i = 0; i < sizeof ctor / sizeof ctor[0]; ++i) {
         if (strcmp(type, ctor[i].a) == 0 || (ctor[i].b && strcmp(type, ctor[i].b) == 0)) {

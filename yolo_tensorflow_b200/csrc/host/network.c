@@ -248,7 +248,7 @@ int resize_network(network *net, int w, int h)
     for (int i = 0; i < net->n; ++i) {
         LAYER_TYPE t = net->layers[i].type;
         if (t != CONVOLUTIONAL && t != MAXPOOL && t != UPSAMPLE && t != REORG && t != SHORTCUT && t != ROUTE && t != YOLO &&
-            t != REGION && t != DROPOUT) {
+            t != REGION && t != DROPOUT && t != AVGPOOL && t != COST) {        /* [softmax]: no branch in the reference either */
             fprintf(stderr, "Cannot resize this type of layer\n");
             return -1;
         }
@@ -304,11 +304,17 @@ int resize_network(network *net, int w, int h)
         case DROPOUT:
             l->w = l->out_w = cw; l->h = l->out_h = ch;
             break;
+        case AVGPOOL:                                       /* resize_avgpool_layer */
+            l->w = cw; l->h = ch;
+            break;
+        case COST:                                          /* resize_cost_layer */
+            l->inputs = l->outputs = net->layers[i - 1].outputs;
+            break;
         default:
             fprintf(stderr, "Cannot resize this type of layer\n");      /* network.c:428 (local/connected/detection) */
             return -1;
         }
-        if (l->type != ROUTE) {
+        if (l->type != ROUTE && l->type != COST) {
             l->inputs = l->w * l->h * l->c;
             l->outputs = l->out_w * l->out_h * l->out_c;
             if (l->type == SHORTCUT) l->inputs = l->outputs;

@@ -127,6 +127,11 @@ lib.b200_comm_init.argtypes = [c_void_p, c_void_p, c_int, c_int]; lib.b200_comm_
 lib.b200_comm_broadcast_weights.argtypes = [c_void_p, c_int]; lib.b200_comm_broadcast_weights.restype = c_int
 lib.b200_comm_set_gather.argtypes = [c_void_p, c_int, c_int, c_int]; lib.b200_comm_set_gather.restype = c_int
 lib.b200_comm_destroy.argtypes = [c_void_p]
+lib.b200_classify_batch.argtypes = [c_void_p, c_void_p, c_int, POINTER(c_int), POINTER(c_float)]; lib.b200_classify_batch.restype = c_int
+lib.b200_classify_submitted.argtypes = [c_void_p, c_void_p, c_int, POINTER(c_int), POINTER(c_float)]
+lib.b200_classify_submitted.restype = c_int
+lib.b200_top_k_arrays.argtypes = [POINTER(c_float), c_int, c_int, c_int, POINTER(c_int)]
+lib.top_k.argtypes = [POINTER(c_float), c_int, c_int, POINTER(c_int)]
 lib.b200_nms_sort_arrays.argtypes = [POINTER(c_float), POINTER(c_float), c_int, c_int, c_float]
 lib.b200_nms_obj_arrays.argtypes = [POINTER(c_float), POINTER(c_float), c_int, c_float, POINTER(c_ubyte)]
 
@@ -310,6 +315,29 @@ class Network:
         return rec, np.array(list(counts))
 
 
+    def classify_batch(self, x, top=5):
+        """b200_classify_batch: x host float32 [batch, c, h, w], or None for the resident device input.  Returns
+        (classes [batch, top] int32, probs [batch, top] float32): top_k of each image's probabilities, on the device."""
+        classes = np.zeros((self.batch, top), np.int32)
+        probs = np.zeros((self.batch, top), np.float32)
+        xp = None
+        if x is not None:
+            x = np.ascontiguousarray(x, dtype=np.float32)
+            xp = x.ctypes.data_as(c_void_p)
+        n = lib.b200_classify_batch(self.ptr, xp, top, classes.ctypes.data_as(POINTER(c_int)), _fptr(probs))
+        if n < 0:
+            raise ValueError("b200_classify_batch refused the network or top=%d (see stderr)" % top)
+        return classes, probs
+
+
+def top_k_arrays(probs, top):
+    """b200_top_k_arrays: the device top-k of every row of probs [rows, n] (top_k of utils.c per row) -> [rows, top] int32"""
+    probs = np.ascontiguousarray(probs, np.float32)
+    out = np.zeros((probs.shape[0], top), np.int32)
+    lib.b200_top_k_arrays(_fptr(probs), probs.shape[0], probs.shape[1], top, out.ctypes.data_as(POINTER(c_int)))
+    return out
+
+
 def dets_to_arrays(dets, n, classes):
     """DETECTION* -> (boxes [n,4], objectness [n], probs [n,classes]) numpy copies"""
     boxes = np.zeros((n, 4), np.float32); obj = np.zeros(n, np.float32); probs = np.zeros((n, classes), np.float32)
@@ -346,4 +374,15 @@ def detect(net, meta, image, thresh=.5, hier_thresh=.5, nms=.45):
     res = sorted(res, key=lambda x: -x[1])
     free_image(im)
     free_detections(dets, num)
+    return res
+
+
+def classify(net, meta, im):
+    """python/darknet.py classify, unchanged semantics: network_predict_image, then every class with its probability,
+    most probable first."""
+    out = predict_image(net, im)
+    res = []
+    for i in range(meta.classes):
+        res.append((meta.names[i], out[i]))
+    res = sorted(res, key=lambda x: -x[1])
     return res

@@ -117,6 +117,10 @@ def walk_shapes(cfg_path):
             L.update(out=(int(o["output"]), 1, 1), bn=int(o.get("batch_normalize", 0)))
         elif t in ("yolo", "region", "detection"):
             L.update(out=(c, h, w), outputs=inputs)
+        elif t in ("avgpool", "avg"):
+            L.update(out=(c, 1, 1))
+        elif t in ("softmax", "soft", "cost"):
+            L.update(out=(c, h, w), outputs=inputs)
         else:
             raise ValueError(f"layer type {t} is outside the YOLO inference path")
         c, h, w = L["out"]
@@ -130,12 +134,13 @@ def walk_shapes(cfg_path):
 # weights
 # --------------------------------------------------------------------------------------------------
 def _head_feeders(layers):
-    """indices of the conv / connected layers whose output is consumed by a detection head"""
+    """indices of the conv / connected layers whose output is consumed by a detection head or, directly or through
+    [avgpool], by a classifier's [softmax]"""
     feed = {}
     for L in layers:
-        if L["type"] in ("yolo", "region", "detection"):
+        if L["type"] in ("yolo", "region", "detection", "softmax", "soft"):
             j = L["index"] - 1
-            while layers[j]["type"] == "dropout":
+            while layers[j]["type"] in ("dropout", "avgpool", "avg"):
                 j -= 1
             feed[j] = L
     return feed
@@ -149,8 +154,14 @@ HEAD_RAW_STD = {
     "yolov3": [410826.0, 431648.0, 582677.0],
     "yolov2": [4.011],
     "yolov1": [11.266],
+    # classifiers: std of the [softmax] input (the logits) with the undamped file, computed on the CPU with the numpy port
+    # (seed-1000 image at the cfg's size; `python tests/np_classifier.py --calibrate darknet53` prints them; the reference
+    # build is not part of this repository, and the port is pinned to it on the detection models)
+    "darknet19": [3.126],
+    "darknet53": [213053.0],
 }
 HEAD_TARGET_STD = 1.5      # logits ~ N(0, 1.5^2)
+CLASSIFIER_TARGET_STD = 2.0   # classifier logits ~ N(0, 2^2): a top-1 probability well inside (0, 1), not one-hot
 # objectness-channel bias per model, tuned (with the reference CPU build, seed-0 weights) so that a realistic
 # 10^1-10^2 anchors per image pass objectness 0.5: yolov3-416 ~230 of 10647, yolov3-tiny ~90 of 2535, yolov2 ~70 of 845
 HEAD_OBJ_BIAS = {"yolov3-tiny": -1.2, "yolov3": -3.0, "yolov2": -0.5}
@@ -189,7 +200,12 @@ def write_weights(cfg_path, out_path, seed=0, damp_heads=True, head_gain=None):
                 n, k = L["n"], L["size"] * L["size"] * L["c"]
                 bias = rng.normal(0, 0.1, n)
                 wts = rng.normal(0, np.sqrt(2.0 / k), (n, k))
-                if L["index"] in feeders:
+                if L["index"] in feeders and feeders[L["index"]]["type"] in ("softmax", "soft"):
+                    if head_gain is not None:
+                        wts *= head_gain
+                    elif raw_std:
+                        wts *= CLASSIFIER_TARGET_STD / raw_std[feeder_rank[L["index"]]]
+                elif L["index"] in feeders:
                     head = feeders[L["index"]]
                     if head_gain is not None:
                         wts *= head_gain
@@ -236,3 +252,4 @@ def _damp_factor(layers, idx):
 def make_images(batch, c, h, w, seed):
     """fp32 NCHW U[0,1) (SURVEY §8d: seed = 1000 + config index)"""
     return np.random.default_rng(seed).random((batch, c, h, w), dtype=np.float32)
+
