@@ -162,6 +162,8 @@ int b200_letterbox_batch_u8(network *net, const unsigned char *const *images, co
 int b200_letterbox_batch(network *net, const image *images, int n);                                                            /* darknet images (fp32 CHW) */
 void b200_fetch_input(network *net, float *dst, int images);      /* the device input buffer as host fp32 NCHW (inspection) */
 
+/* network_predict + get_network_boxes + do_nms_sort for every image of the batch.  input: host fp32 NCHW, or NULL /
+ * B200_INPUT_RESIDENT for what the device input buffer holds (e.g. after b200_letterbox_batch_u8). */
 int b200_detect_batch(network *net, const float *input, int w, int h, float thresh, float nms_thresh,
                       int relative, b200_det *out, int max_out, int *counts);
 

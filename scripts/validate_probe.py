@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Throughput of the batched validate_detector driver (b200_validate_images: device letterbox -> forward -> decode/NMS ->
 result file) on YOLOv3-416, batch 64, over decoded 640x480 images held in host memory.
-Usage: python scripts/validate_probe.py [images]      (B200_LETTERBOX_SYNC=1: uploads on the compute stream, for comparison)"""
+Usage: python scripts/validate_probe.py [images]"""
 import os, sys, tempfile, time
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -23,6 +23,5 @@ net.validate_images(images[:128], paths[:128], "coco", out, thresh=.5)       # w
 t = time.perf_counter()
 n = net.validate_images(images, paths, "coco", out, thresh=.5)
 dt = time.perf_counter() - t
-print("validate_images: %d images, %d records, %.1f ms, %.0f images/s (%s)" %
-      (m, n, dt * 1e3, m / dt, "uploads on the compute stream" if os.environ.get("B200_LETTERBOX_SYNC") else "uploads on the copy stream"))
+print("validate_images: %d images, %d records, %.1f ms, %.0f images/s" % (m, n, dt * 1e3, m / dt))
 net.close()

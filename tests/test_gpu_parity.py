@@ -945,6 +945,23 @@ def test_resident_input_serving_loop(dn, workdir):
     net.close()
 
 
+def test_detect_batch_takes_the_resident_input_sentinel(dn, workdir):
+    """b200_detect_batch with B200_INPUT_RESIDENT reads the device input buffer, like NULL, as b200_classify_batch does"""
+    net, _, _ = open_net(dn, "yolov3-tiny", 3, 160, workdir, dn.PREC_BF16)
+    rng = np.random.default_rng(23)
+    images = [rng.integers(0, 256, (140 + 11 * i, 210 - 13 * i, 3), dtype=np.uint8) for i in range(3)]
+    order = lambda r: r[np.lexsort((r["cls"], r["box_id"], r["image"]))]
+    assert net.letterbox_batch_u8(images) == 0
+    want, want_counts = net.detect_batch(None, 0, 0, .3, .45, relative=0)
+    assert len(want) > 0
+    out = (dn.B200_DET * 100000)(); counts = (ctypes.c_int * 3)()
+    assert net.letterbox_batch_u8(images) == 0
+    n = dn.lib.b200_detect_batch(net.ptr, ctypes.c_void_p(1), 0, 0, .3, .45, 0, out, 100000, counts)
+    assert n == len(want) and list(counts) == want_counts.tolist()
+    assert order(np.ctypeslib.as_array(out)[:n].copy()).tobytes() == order(want).tobytes()
+    net.close()
+
+
 def test_host_input_right_after_letterbox(dn, workdir):
     """the letterbox kernel is asynchronous: a host batch staged right behind it (chunked copies on the copy stream) must
     land after it, not under it"""

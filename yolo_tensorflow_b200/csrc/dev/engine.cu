@@ -122,18 +122,26 @@ static void writers_of(const b200_engine *e, const network *net, int j, std::vec
     out.push_back(j);
 }
 
-static void build_engine_device_state(b200_engine *e, network *net)
+static bool is_detection_head(LAYER_TYPE t) { return t == YOLO || t == REGION || t == DETECTION; }
+
+// the layer whose output network_predict returns: the last one that is not a [cost]
+static int output_layer(const network *net)
+{
+    int last = net->n - 1;
+    while (last > 0 && net->layers[last].type == COST) --last;
+    return last;
+}
+
+// streams and events of the serving loop and the input buffer
+static void create_device_resources(b200_engine *e, const network *net)
 {
     require_device(net->gpu_index);
     B200_CHECK(cudaGetDevice(&e->device));
     B200_CHECK(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
     B200_CHECK(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
     for (auto &ev : e->copy_done) B200_CHECK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-    const int esize = (int)dt_size(e->act_dtype);
-    auto cons = consumers_of(net);
-
     e->d_input = (float *)dev_alloc((size_t)e->cap * net->inputs * sizeof(float));
-    e->d_input_next = nullptr;                                    // allocated on the first b200_submit_batch
+    // d_input_next is allocated on the first b200_submit_batch
     B200_CHECK(cudaEventCreateWithFlags(&e->submit_done, cudaEventDisableTiming));
     B200_CHECK(cudaStreamCreateWithFlags(&e->d2h_stream, cudaStreamNonBlocking));
     B200_CHECK(cudaEventCreateWithFlags(&e->tail_done, cudaEventDisableTiming));
@@ -141,11 +149,12 @@ static void build_engine_device_state(b200_engine *e, network *net)
     B200_CHECK(cudaEventCreateWithFlags(&e->fwd_done, cudaEventDisableTiming));
     B200_CHECK(cudaEventCreateWithFlags(&e->lb_uploaded, cudaEventDisableTiming));
     B200_CHECK(cudaEventCreateWithFlags(&e->lb_done, cudaEventDisableTiming));
-    e->fwd_enqueued = 0;
-    e->submitted = 0;
-    size_t max_floats = (size_t)e->cap * net->inputs;
+}
 
-    // ---- shortcut fusion: conv -> shortcut pairs whose add can ride in the conv epilogue --------------
+// fused_into / fused_away, block_head, up_fused / up_away: the layers whose work rides in a neighbouring kernel
+static void plan_fusions(b200_engine *e, const network *net, const std::vector<std::vector<int>> &cons)
+{
+    // shortcut fusion: conv -> shortcut pairs whose add can ride in the conv epilogue
     for (int i = 1; i + 1 < net->n; ++i) {
         const layer &c = net->layers[i], &sc = net->layers[i + 1];
         if (!e->fusion || e->precision != B200_PREC_BF16) break;
@@ -156,12 +165,12 @@ static void build_engine_device_state(b200_engine *e, network *net)
         if (c.size == 1 && (c.stride != 1 || c.pad != 0)) continue;
         if (!conv_tc_shape_supported(c.c, c.stride, act_id(c.activation)) || c.out_c % 16 != 0) continue;
         LAYER_TYPE src = net->layers[sc.index].type;
-        if (src == YOLO || src == REGION || src == DETECTION || src == CONNECTED) continue;
+        if (is_detection_head(src) || src == CONNECTED) continue;
         e->L[i].fused_into = i + 1;
         e->L[i + 1].fused_away = true;
     }
 
-    // ---- fused residual blocks: 1x1 (64 -> 32) -> 3x3 (32 -> 64) -> shortcut from the block input, in ONE kernel ----------
+    // fused residual blocks: 1x1 (64 -> 32) -> 3x3 (32 -> 64) -> shortcut from the block input, in ONE kernel
     for (int i = 1; i + 2 < net->n; ++i) {
         const layer &c1 = net->layers[i], &c2 = net->layers[i + 1], &sc = net->layers[i + 2];
         if (c1.type != CONVOLUTIONAL || c2.type != CONVOLUTIONAL || sc.type != SHORTCUT) continue;
@@ -173,7 +182,7 @@ static void build_engine_device_state(b200_engine *e, network *net)
         e->L[i].block_head = true;
     }
 
-    // ---- conv -> [upsample] (stride 2, scale 1): the conv's store warp writes the four copies itself -----------------------
+    // conv -> [upsample] (stride 2, scale 1): the conv's store warp writes the four copies itself
     for (int i = 1; i + 1 < net->n && e->fusion && e->precision == B200_PREC_BF16 && !getenv("B200_NO_UPSAMPLE_FUSION"); ++i) {
         const layer &c = net->layers[i], &u = net->layers[i + 1];
         if (c.type != CONVOLUTIONAL || u.type != UPSAMPLE || u.stride != 2 || u.reverse || u.scale != 1.f) continue;
@@ -183,11 +192,18 @@ static void build_engine_device_state(b200_engine *e, network *net)
         e->L[i].up_fused = true;
         e->L[i + 1].up_away = true;
     }
+}
 
-    // ---- zero-copy concatenation: a route's inputs are produced straight into channel slices of the route's buffer ----
-    // (route_layer.c:80-95 copies every input; here only inputs that cannot be placed are copied).  An input is placed
-    // when its producer writes through a TView (row pitch = the route's channel count) and nothing needs it dense.
-    std::vector<int> place_route(net->n, -1), place_off(net->n, 0);
+// zero-copy concatenation: a route's inputs are produced straight into channel slices of the route's buffer
+// (route_layer.c:80-95 copies every input; here only inputs that cannot be placed are copied).  An input is placed
+// when its producer writes through a TView (row pitch = the route's channel count) and nothing needs it dense.
+// place_route[j] = the route layer j's output is placed in (or -1), place_off[j] = its first channel there.
+static void plan_route_placement(const b200_engine *e, const network *net, const std::vector<std::vector<int>> &cons,
+                                 std::vector<int> &place_route, std::vector<int> &place_off)
+{
+    const int esize = (int)dt_size(e->act_dtype);
+    place_route.assign(net->n, -1);
+    place_off.assign(net->n, 0);
     for (int r = 0; r < net->n && !getenv("B200_NO_ZERO_COPY_ROUTE"); ++r) {
         const layer &rl = net->layers[r];
         if (rl.type != ROUTE || rl.n < 2 || rl.out_c == 0) continue;
@@ -202,12 +218,19 @@ static void build_engine_device_state(b200_engine *e, network *net)
             if (sl.type == CONVOLUTIONAL && e->L[sidx].fused_into >= 0) ok = false;
             for (int c : cons[sidx]) {
                 LAYER_TYPE ct = net->layers[c].type;
-                if (ct == CONNECTED || ct == YOLO || ct == REGION || ct == DETECTION) ok = false;     // these read dense buffers
+                if (ct == CONNECTED || is_detection_head(ct)) ok = false;     // these read dense buffers
             }
             if (ok) { place_route[sidx] = r; place_off[sidx] = coff; }
             coff += sl.out_c;
         }
     }
+}
+
+// the classifier tail (cls_layer, cls_logits), every layer's output view and the fp32 transfer scratch, and the first
+// layer's input (stem, in_view)
+static void plan_outputs(b200_engine *e, const network *net, const std::vector<std::vector<int>> &cons,
+                         const std::vector<int> &place_route, const std::vector<int> &place_off)
+{
     auto concat_slice = [&](int sidx, const layer &sl, int dtype) -> TView {
         const int r = place_route[sidx];
         DevLayer &rd = e->L[r];
@@ -219,19 +242,15 @@ static void build_engine_device_state(b200_engine *e, network *net)
         return TView{(unsigned char *)rd.out.p + (size_t)place_off[sidx] * dt_size(dtype), e->cap, sl.out_h, sl.out_w, sl.out_c, rl.out_c, dtype};
     };
 
-    // ---- classifier tail: the [softmax] the network ends in, and the convolution feeding it (directly or through [avgpool]) ----
+    // classifier tail: the [softmax] the network ends in, and the convolution feeding it (directly or through [avgpool])
     auto only_consumer_is = [&](int j, LAYER_TYPE t) { return j + 1 < net->n && cons[j].size() == 1 && cons[j][0] == j + 1 && net->layers[j + 1].type == t; };
-    e->cls_layer = -1;
-    {
-        int last = net->n - 1;
-        while (last > 0 && net->layers[last].type == COST) --last;
-        if (net->layers[last].type == SOFTMAX) e->cls_layer = last;
-    }
+    if (net->layers[output_layer(net)].type == SOFTMAX) e->cls_layer = output_layer(net);
     for (int i = 0; i < net->n; ++i)
         e->L[i].cls_logits = net->layers[i].type == CONVOLUTIONAL &&
                              (only_consumer_is(i, SOFTMAX) || (only_consumer_is(i, AVGPOOL) && only_consumer_is(i + 1, SOFTMAX)));
 
-    // ---- output views ------------------------------------------------------------------------------
+    // output views
+    size_t max_floats = (size_t)e->cap * net->inputs;
     for (int i = 0; i < net->n; ++i) {
         const layer &l = net->layers[i];
         DevLayer &d = e->L[i];
@@ -303,15 +322,19 @@ static void build_engine_device_state(b200_engine *e, network *net)
     e->xfer_floats = max_floats;
     e->xfer = (float *)dev_alloc(max_floats * sizeof(float));
 
-    // ---- first layer input -------------------------------------------------------------------------------
+    // first layer input
     const layer &l0 = net->layers[0];
     e->L[0].stem = (l0.type == CONVOLUTIONAL && l0.c <= 4);
     if (!e->L[0].stem) {
         if (!(net->h && net->w && net->c)) { fprintf(stderr, "b200-darknet: network input must be an image\n"); abort(); }
-        e->in_view = TView{dev_alloc((size_t)e->cap * net->inputs * esize), e->cap, net->h, net->w, net->c, net->c, e->act_dtype};
+        e->in_view = TView{dev_alloc((size_t)e->cap * net->inputs * dt_size(e->act_dtype)), e->cap, net->h, net->w, net->c, net->c, e->act_dtype};
     }
+}
 
-    // ---- parameter arena -----------------------------------------------------------------------------------
+// the parameter arena: every layer's weight / scale / shift / bias offsets, then the arena itself (zeroed)
+static void plan_arena(b200_engine *e, const network *net)
+{
+    const int esize = (int)dt_size(e->act_dtype);
     size_t off = 0;
     for (int i = 0; i < net->n; ++i) {
         const layer &l = net->layers[i];
@@ -345,8 +368,11 @@ static void build_engine_device_state(b200_engine *e, network *net)
         if (l.type == CONVOLUTIONAL || l.type == CONNECTED) { d.scale = (float *)(e->arena + d.scale_off); d.shift = (float *)(e->arena + d.shift_off); }
         if (l.type == LOCAL) { d.lbias = (float *)(e->arena + d.lbias_off); d.scale = (float *)(e->arena + d.scale_off); }
     }
+}
 
-    // ---- kernel selection ------------------------------------------------------------------------------------
+// every layer's kernel and tcgen05 plan; a fusion whose shapes the plan does not take is undone here
+static void select_kernels(b200_engine *e, const network *net, const std::vector<std::vector<int>> &cons, const std::vector<int> &place_route)
+{
     for (int i = 0; i < net->n; ++i) {
         const layer &l = net->layers[i];
         DevLayer &d = e->L[i];
@@ -425,7 +451,7 @@ static void build_engine_device_state(b200_engine *e, network *net)
         case DROPOUT: d.kernel = "alias"; break;
         case LOCAL:
             d.kernel = "local";
-            if (e->precision == B200_PREC_BF16 && !getenv("B200_LOCAL_SIMT")) {
+            if (e->precision == B200_PREC_BF16) {
                 // 49 independent GEMMs [images x 9C] x [9C x filters]: the conv kernel with one pixel per tile and the weight
                 // box taken from that pixel's own slab
                 ConvParams p{l.size, l.stride, l.pad, act_id(l.activation), d.w, d.scale, d.lbias, l.n};
@@ -436,8 +462,7 @@ static void build_engine_device_state(b200_engine *e, network *net)
         case CONNECTED: {
             d.kernel = "connected";
             const DevLayer &pd = e->L[i - 1];
-            if (e->precision == B200_PREC_BF16 && !getenv("B200_CONNECTED_SIMT") && pd.out.dtype == DT_BF16 && pd.out.ld == pd.out.c &&
-                l.inputs % 64 == 0) {
+            if (e->precision == B200_PREC_BF16 && pd.out.dtype == DT_BF16 && pd.out.ld == pd.out.c && l.inputs % 64 == 0) {
                 // out[b][o] = sum_i in[b][i] W[o][i] is a 1x1 convolution over a 1 x 1 "image" with `inputs` channels
                 d.fc_tmp = (float *)dev_alloc((size_t)e->cap * d.cout_pad * sizeof(float));
                 TView fin{pd.out.p, e->cap, 1, 1, l.inputs, l.inputs, DT_BF16};
@@ -458,8 +483,11 @@ static void build_engine_device_state(b200_engine *e, network *net)
         default: break;
         }
     }
+}
 
-    // ---- flows: maximal runs of flow-capable convolutions (nothing else launching in between) become ONE persistent kernel ----
+// flows: maximal runs of flow-capable convolutions (nothing else launching in between) become ONE persistent kernel
+static void plan_flows(b200_engine *e, const network *net)
+{
     e->flow_at.assign(net->n, -1);
     e->flow_on = 1;
     for (int i = 1; i < net->n && e->precision == B200_PREC_BF16;) {
@@ -499,13 +527,16 @@ static void build_engine_device_state(b200_engine *e, network *net)
         }
         i = restart_here ? j : j + 1;
     }
+}
 
-    // ---- heads for decode ---------------------------------------------------------------------------------------
+// the decode's head descriptors (host and device copies), tail_guard_layer, and the page-locked host outputs
+static void plan_heads(b200_engine *e, const network *net)
+{
     int base = 0;
-    e->raw_decode_ok = !getenv("B200_NO_RAW_DECODE");
+    e->raw_decode_ok = true;
     for (int i = 0; i < net->n; ++i) {
         const layer &l = net->layers[i];
-        if (l.type != YOLO && l.type != REGION && l.type != DETECTION) continue;
+        if (!is_detection_head(l.type)) continue;
         HeadDesc h;
         memset(&h, 0, sizeof h);
         h.type = l.type; h.w = l.w; h.h = l.h; h.n = l.n; h.classes = l.classes; h.coords = l.coords;
@@ -554,57 +585,59 @@ static void build_engine_device_state(b200_engine *e, network *net)
     // that overwrites a buffer the tail reads — a head's l.output or the logits of the convolution feeding it — waits for it
     e->tail_guard_layer = net->n;
     for (int i = 0; i < net->n; ++i) {
-        const LAYER_TYPE t = net->layers[i].type;
-        if (t != YOLO && t != REGION && t != DETECTION) continue;
+        if (!is_detection_head(net->layers[i].type)) continue;
         int feeder = i > 0 ? i - 1 : 0;                      // the layer whose output the head (and the raw-logit decode) reads
         while (feeder > 0 && net->layers[feeder].type == DROPOUT) --feeder;
         if (feeder < e->tail_guard_layer) e->tail_guard_layer = feeder;
     }
     // the reference API moves the heads' l.output between host and device on every call (network.c:505, yolo_layer.c:359-362
     // on the way out; get_network_boxes reads them on the way in): page-lock those host buffers while this plan lives
-    {
-        int last = net->n - 1;
-        while (last > 0 && net->layers[last].type == COST) --last;
-        for (int i = 0; i < net->n; ++i) {
-            const layer &l = net->layers[i];
-            const bool head = l.type == YOLO || l.type == REGION || l.type == DETECTION;
-            if ((!head && i != last) || !l.output || l.type == DROPOUT) continue;
-            if (cudaHostRegister(l.output, (size_t)e->cap * l.outputs * sizeof(float), cudaHostRegisterDefault) == cudaSuccess) e->pinned_host.push_back(l.output);
-            else cudaGetLastError();                       // not fatal: the copies just stay pageable
-        }
+    const int last = output_layer(net);
+    for (int i = 0; i < net->n; ++i) {
+        const layer &l = net->layers[i];
+        if ((!is_detection_head(l.type) && i != last) || !l.output || l.type == DROPOUT) continue;
+        if (cudaHostRegister(l.output, (size_t)e->cap * l.outputs * sizeof(float), cudaHostRegisterDefault) == cudaSuccess) e->pinned_host.push_back(l.output);
+        else cudaGetLastError();                       // not fatal: the copies just stay pageable
     }
     if (!e->heads.empty()) {
         e->d_heads = (HeadDesc *)dev_alloc(e->heads.size() * sizeof(HeadDesc));
         B200_CHECK(cudaMemcpy(e->d_heads, e->heads.data(), e->heads.size() * sizeof(HeadDesc), cudaMemcpyHostToDevice));
     }
+}
+
+// the plan: each pass reads the decisions of the passes before it
+static void build_engine_device_state(b200_engine *e, network *net)
+{
+    create_device_resources(e, net);
+    const auto cons = consumers_of(net);
+    plan_fusions(e, net, cons);
+    std::vector<int> place_route, place_off;
+    plan_route_placement(e, net, cons, place_route, place_off);
+    plan_outputs(e, net, cons, place_route, place_off);
+    plan_arena(e, net);
+    select_kernels(e, net, cons, place_route);
+    plan_flows(e, net);
+    plan_heads(e, net);
     g_cuda_ready = true;
 }
 
-extern "C" b200_engine *b200_engine_create(network *net, int precision)
+static b200_engine *engine_create(network *net, int precision, int fusion)
 {
     b200_engine *e = new b200_engine();
     e->precision = precision;
     e->act_dtype = precision == B200_PREC_FP32 ? DT_F32 : DT_BF16;
     e->n = net->n;
     e->cap = net->batch;
-    e->conv_backend = 0;
-    e->head_sync = 1;
+    e->fusion = fusion;
     e->L.resize(net->n);
-    for (auto &d : e->L) { d = DevLayer(); d.tc = nullptr; d.head_out = nullptr; d.w = nullptr; d.stem = false; d.owns_out = false; d.fused_into = -1; d.fused_away = false; d.block_head = false; d.up_fused = false; d.up_away = false; d.fc_tmp = nullptr; d.pool_fused = false; d.pool_away = false; d.reorg_table = nullptr; d.cls_logits = false; }
-    e->fusion = b200_get_default_fusion();
-    e->stream = nullptr; e->d_input = nullptr; e->d_input_next = nullptr; e->submitted = 0; e->arena = nullptr; e->xfer = nullptr; e->d_heads = nullptr;
-    e->in_view = TView{nullptr, 0, 0, 0, 0, 0, 0};
-    memset(&e->cand, 0, sizeof e->cand); e->cand_slots = 0;
-    memset(&e->nms_scratch, 0, sizeof e->nms_scratch);
-    e->d_records = nullptr; e->records_cap = 0; e->d_record_count = nullptr; e->comm = nullptr;
-    e->d_raw = nullptr; e->raw_cap = 0; e->d_lb_items = nullptr; e->d_im_dims[0] = e->d_im_dims[1] = nullptr; e->dims_cur = 0; e->dims_pending = 0;
-    e->h_box = e->h_obj = e->h_prob = nullptr; e->h_id = nullptr; e->h_cap = 0;
-    e->boxes_per_image = 0; e->classes = 0; e->has_tree = false; e->d_map = nullptr;
-    e->cls_layer = -1; e->d_top_cls = nullptr; e->d_top_prob = nullptr;
     // Parsing a cfg (layer table, shapes) works on a machine without a GPU; anything that computes does not.
     if (cuda_usable()) build_engine_device_state(e, net);
-    else e->device = -1;
     return e;
+}
+
+extern "C" b200_engine *b200_engine_create(network *net, int precision)
+{
+    return engine_create(net, precision, b200_get_default_fusion());
 }
 
 static void need_device(const b200_engine *e, const char *what)
@@ -741,10 +774,7 @@ extern "C" b200_engine *b200_engine_recreate(b200_engine *old, network *net)
     B200Comm *comm = old->comm;                 // the communicator belongs to the process, not to the plan
     old->comm = nullptr;
     b200_engine_destroy(old);
-    const int default_fusion = b200_get_default_fusion();
-    b200_set_default_fusion(fusion);
-    b200_engine *e = b200_engine_create(net, precision);
-    b200_set_default_fusion(default_fusion);
+    b200_engine *e = engine_create(net, precision, fusion);
     e->head_sync = head_sync;
     e->comm = comm;
     if (e->device >= 0) b200_engine_upload_weights(e, net);
@@ -914,22 +944,24 @@ static int stage_input(b200_engine *e, network *net, const float *input)
     return 1;
 }
 
+// enqueue the copy of layer i's output (the first `batch` images, fp32 NCHW) to host memory at dst on the compute stream
+static void copy_layer_to_host(b200_engine *e, const network *net, int i, int batch, float *dst)
+{
+    const size_t bytes = (size_t)batch * net->layers[i].outputs * sizeof(float);
+    if (e->L[i].head_out) {
+        B200_CHECK(cudaMemcpyAsync(dst, e->L[i].head_out, bytes, cudaMemcpyDeviceToHost, e->stream));
+    } else {
+        launch_view_to_nchw_f32(view_of(e->L[i], batch), e->xfer, e->stream);
+        B200_CHECK(cudaMemcpyAsync(dst, e->xfer, bytes, cudaMemcpyDeviceToHost, e->stream));
+    }
+}
+
 static void sync_heads_to_host(b200_engine *e, network *net)
 {
-    int batch = logical_batch(e, net);
-    int last = net->n - 1;
-    while (last > 0 && net->layers[last].type == COST) --last;
-    for (int i = 0; i < net->n; ++i) {
-        const layer &l = net->layers[i];
-        bool head = l.type == YOLO || l.type == REGION || l.type == DETECTION;
-        if (!head && i != last) continue;
-        if (e->L[i].head_out) {
-            B200_CHECK(cudaMemcpyAsync(l.output, e->L[i].head_out, (size_t)batch * l.outputs * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
-        } else {
-            launch_view_to_nchw_f32(view_of(e->L[i], batch), e->xfer, e->stream);
-            B200_CHECK(cudaMemcpyAsync(l.output, e->xfer, (size_t)batch * l.outputs * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
-        }
-    }
+    const int batch = logical_batch(e, net);
+    const int last = output_layer(net);
+    for (int i = 0; i < net->n; ++i)
+        if (is_detection_head(net->layers[i].type) || i == last) copy_layer_to_host(e, net, i, batch, net->layers[i].output);
 }
 
 extern "C" void b200_engine_forward(b200_engine *e, network *net, const float *input)
@@ -945,6 +977,33 @@ extern "C" void b200_engine_forward_resident(b200_engine *e, network *net)
 {
     need_device(e, "network_predict");
     forward_layers(e, net, 0, net->n);
+}
+
+// with head sync off nobody reads l.output of the heads: the batched detection path skips forward_yolo_layer and decodes from
+// the head convolutions' fp32 logits (identical arithmetic: the logistic is evaluated on the fly for the objectness test and for
+// survivors).  Never for a classifier, which has no heads.
+static bool use_raw_decode(const b200_engine *e) { return !e->head_sync && e->raw_decode_ok && !e->heads.empty(); }
+
+// the sizes recorded by the last b200_letterbox_batch* call belong to the batch whose forward pass is enqueued next
+static void adopt_letterbox_dims(b200_engine *e)
+{
+    if (e->dims_pending) { e->dims_cur ^= 1; e->dims_pending = 0; }
+}
+
+// enqueue the current batch's forward pass from layer `first`: 0, 1 after the chunked stage_input, or net->n when it is
+// already in the stream
+static void enqueue_forward(b200_engine *e, network *net, int first)
+{
+    if (first >= net->n) return;
+    adopt_letterbox_dims(e);
+    forward_layers(e, net, first, net->n, use_raw_decode(e));
+}
+
+// `input` of the batch entry points: NULL or B200_INPUT_RESIDENT is the device input buffer as it stands, anything else a
+// host batch to stage.  Returns the first layer still to run.
+static int stage_batch_input(b200_engine *e, network *net, const float *input)
+{
+    return (input && input != B200_INPUT_RESIDENT) ? stage_input(e, net, input) : 0;
 }
 
 extern "C" float *b200_engine_input_device(b200_engine *e) { return e->d_input; }
@@ -999,26 +1058,16 @@ extern "C" const char *b200_flow_desc(network *net, int k, int *first, int *last
 // ----------------------------------------------------------------------------------------------------
 static void need_materialised(const b200_engine *e, int i)
 {
-    if (e->L[i].block_head) {
-        fprintf(stderr, "b200-darknet: layer %d's output is not materialised: it is computed inside the fused residual block kernel of layer %d. "
-                        "Parse with B200_FUSE=0 (or b200_set_default_fusion(0)) to inspect it.\n", i, i + 1);
-        abort();
-    }
-    if (e->L[i].pool_fused) {
-        fprintf(stderr, "b200-darknet: layer %d's output is not materialised: the stem kernel stores it max-pooled into layer %d's buffer. "
-                        "Parse with B200_FUSE=0 (or b200_set_default_fusion(0)) to inspect it.\n", i, i + 1);
-        abort();
-    }
-    if (e->L[i].up_fused) {
-        fprintf(stderr, "b200-darknet: layer %d's output is not materialised: it is written upsampled into layer %d's buffer. "
-                        "Parse with B200_FUSE=0 (or b200_set_default_fusion(0)) to inspect it.\n", i, i + 1);
-        abort();
-    }
-    if (e->L[i].fused_into >= 0) {
-        fprintf(stderr, "b200-darknet: layer %d's output is not materialised: its shortcut (layer %d) is fused into the conv epilogue. "
-                        "Parse with B200_FUSE=0 (or b200_set_default_fusion(0)) to inspect it.\n", i, e->L[i].fused_into);
-        abort();
-    }
+    const DevLayer &d = e->L[i];
+    const char *why = d.block_head   ? "it is computed inside the fused residual block kernel of the next layer"
+                    : d.pool_fused   ? "the stem kernel stores it max-pooled into the next layer's buffer"
+                    : d.up_fused     ? "it is written upsampled into the next layer's buffer"
+                    : d.fused_into >= 0 ? "its shortcut is fused into the conv epilogue"
+                    : nullptr;
+    if (!why) return;
+    fprintf(stderr, "b200-darknet: layer %d's output is not materialised: %s. "
+                    "Parse with B200_FUSE=0 (or b200_set_default_fusion(0)) to inspect it.\n", i, why);
+    abort();
 }
 
 extern "C" void b200_fetch_layer_output(network *net, int i, float *out)
@@ -1026,14 +1075,7 @@ extern "C" void b200_fetch_layer_output(network *net, int i, float *out)
     b200_engine *e = b200_engine_of(net);
     need_device(e, "b200_fetch_layer_output");
     need_materialised(e, i);
-    int batch = logical_batch(e, net);
-    size_t bytes = (size_t)batch * net->layers[i].outputs * sizeof(float);
-    if (e->L[i].head_out) {
-        B200_CHECK(cudaMemcpyAsync(out, e->L[i].head_out, bytes, cudaMemcpyDeviceToHost, e->stream));
-    } else {
-        launch_view_to_nchw_f32(view_of(e->L[i], batch), e->xfer, e->stream);
-        B200_CHECK(cudaMemcpyAsync(out, e->xfer, bytes, cudaMemcpyDeviceToHost, e->stream));
-    }
+    copy_layer_to_host(e, net, i, logical_batch(e, net), out);
     B200_CHECK(cudaStreamSynchronize(e->stream));
 }
 
@@ -1047,7 +1089,7 @@ extern "C" void b200_set_layer_output(network *net, int i, const float *in)
     if (e->L[i].head_out) {
         B200_CHECK(cudaMemcpyAsync(e->L[i].head_out, in, bytes, cudaMemcpyHostToDevice, e->stream));
         const layer &l = net->layers[i];                  // the host copy get_network_boxes trusts follows (b200_engine_push_heads)
-        if ((l.type == YOLO || l.type == REGION || l.type == DETECTION) && l.output && l.output != in) memcpy(l.output, in, bytes);
+        if (is_detection_head(l.type) && l.output && l.output != in) memcpy(l.output, in, bytes);
     } else {
         B200_CHECK(cudaMemcpyAsync(e->xfer, in, bytes, cudaMemcpyHostToDevice, e->stream));
         launch_nchw_f32_to_view(e->xfer, view_of(e->L[i], batch), e->stream);
@@ -1147,7 +1189,7 @@ extern "C" void b200_profile_forward(network *net, int iters, float *ms)
     b200_engine *e = b200_engine_of(net);
     need_device(e, "b200_profile_forward");
     const int batch = logical_batch(e, net);
-    const bool skip_yolo = !e->head_sync && e->raw_decode_ok && !e->heads.empty();
+    const bool skip_yolo = use_raw_decode(e);
     if (iters < 1) iters = 1;
     std::vector<cudaEvent_t> ev(2 * (size_t)iters + 1);
     for (auto &x : ev) B200_CHECK(cudaEventCreate(&x));
@@ -1281,7 +1323,7 @@ extern "C" void b200_engine_push_heads(b200_engine *e, network *net, int items)
     if (items > logical_batch(e, net)) items = logical_batch(e, net);
     for (int i = 0; i < net->n; ++i) {
         const layer &l = net->layers[i];
-        if ((l.type != YOLO && l.type != REGION && l.type != DETECTION) || !e->L[i].head_out || !l.output) continue;
+        if (!is_detection_head(l.type) || !e->L[i].head_out || !l.output) continue;
         B200_CHECK(cudaMemcpyAsync(e->L[i].head_out, l.output, (size_t)items * l.outputs * sizeof(float), cudaMemcpyHostToDevice, e->stream));
     }
 }
@@ -1305,12 +1347,6 @@ extern "C" void b200_engine_avg_flipped(b200_engine *e, network *net)
 // forward (from layer `first`; first = net->n: the forward pass is already in the stream) + decode + NMS + collect, all
 // enqueued on the compute stream; `after_tail` (optional) runs once they are enqueued and before the host waits, so that the
 // caller can put the NEXT batch's work behind them; the results then come back on their own stream while that work runs.
-// the sizes recorded by the last b200_letterbox_batch* call belong to the batch whose forward pass is enqueued next
-static void adopt_letterbox_dims(b200_engine *e)
-{
-    if (e->dims_pending) { e->dims_cur ^= 1; e->dims_pending = 0; }
-}
-
 template <typename F>
 static int detect_core(b200_engine *e, network *net, int first, int w, int h, float thresh, float nms_thresh, int relative,
                        b200_det *out, int max_out, int *counts, F after_tail)
@@ -1320,11 +1356,7 @@ static int detect_core(b200_engine *e, network *net, int first, int w, int h, fl
         fprintf(stderr, "b200-darknet: networks with a class tree (YOLO9000) go through get_network_boxes + do_nms_sort; the fused batched path does not take them\n");
         abort();
     }
-    // with head sync off nobody reads l.output of the heads: skip forward_yolo_layer and decode from the head convolutions'
-    // fp32 logits (identical arithmetic: the logistic is evaluated on the fly for the objectness test and for survivors)
-    const int use_raw = (!e->head_sync && e->raw_decode_ok && !e->heads.empty()) ? 1 : 0;
-    if (first < net->n) adopt_letterbox_dims(e);
-    forward_layers(e, net, first, net->n, use_raw != 0);
+    enqueue_forward(e, net, first);
     if (e->heads.empty()) { after_tail(); B200_CHECK(cudaStreamSynchronize(e->stream)); return 0; }
     ensure_candidates(e, e->cap);
     if (e->records_cap < max_out) {
@@ -1338,14 +1370,12 @@ static int detect_core(b200_engine *e, network *net, int first, int w, int h, fl
     if (w == 0 && h == 0 && !im_dims) { fprintf(stderr, "b200-darknet: w = h = 0 needs a preceding b200_letterbox_batch call\n"); abort(); }
     // decode + NMS + collect go to their own stream behind the forward pass: in the serving loop the next batch's forward pass
     // is enqueued right after (after_tail), and these small latency-bound kernels then run beside its first, bandwidth-bound
-    // layers instead of in front of them (B200_NO_TAIL_OVERLAP=1 keeps everything on one stream: the A/B switch)
-    static const bool tail_overlap = getenv("B200_NO_TAIL_OVERLAP") == nullptr;
-    cudaStream_t ts = tail_overlap ? e->tail_stream : e->stream;
-    if (tail_overlap) {
-        B200_CHECK(cudaEventRecord(e->fwd_done, e->stream));
-        B200_CHECK(cudaStreamWaitEvent(ts, e->fwd_done, 0));
-    }
-    launch_decode(e->d_heads, (int)e->heads.size(), 0, batch, net->w, net->h, w, h, thresh, relative, 1, use_raw, e->cand, ts, im_dims);
+    // layers instead of in front of them
+    cudaStream_t ts = e->tail_stream;
+    B200_CHECK(cudaEventRecord(e->fwd_done, e->stream));
+    B200_CHECK(cudaStreamWaitEvent(ts, e->fwd_done, 0));
+    launch_decode(e->d_heads, (int)e->heads.size(), 0, batch, net->w, net->h, w, h, thresh, relative, 1, use_raw_decode(e) ? 1 : 0,
+                  e->cand, ts, im_dims);
     launch_nms_sort(e->cand.box, e->cand.prob, e->cand.obj, e->cand.count, batch, e->cand.cap, e->classes, nms_thresh,
                     e->boxes_per_image, &e->nms_scratch, e->cand.cls_count, ts);
     B200_CHECK(cudaMemsetAsync(e->d_record_count, 0, sizeof(int), ts));
@@ -1395,7 +1425,7 @@ extern "C" int b200_detect_batch(network *net, const float *input, int w, int h,
     b200_engine *e = b200_engine_of(net);
     need_device(e, "b200_detect_batch");
     if (refuse_classifier(e, "b200_detect_batch")) return -1;
-    const int first = input ? stage_input(e, net, input) : 0;
+    const int first = stage_batch_input(e, net, input);
     return detect_core(e, net, first, w, h, thresh, nms_thresh, relative, out, max_out, counts);
 }
 
@@ -1442,19 +1472,14 @@ static int letterbox_batch(network *net, const void *const *images, const int *w
     // previous upload and the kernel was enqueued before the forward pass whose results the caller has meanwhile collected or
     // is about to; the dims slot written is the one of the batch before the one in flight).  Only the letterbox kernel itself
     // joins the compute stream, behind whatever is already there.
-    static const bool lb_sync = getenv("B200_LETTERBOX_SYNC") != nullptr;       // A/B knob: everything on the compute stream
-    cudaStream_t up = lb_sync ? e->stream : e->copy_stream;
-    if (!lb_sync) {                                                               // the previous letterbox kernel must be done with d_raw
-        B200_CHECK(cudaStreamWaitEvent(up, e->lb_done, 0));
-    }
+    cudaStream_t up = e->copy_stream;
+    B200_CHECK(cudaStreamWaitEvent(up, e->lb_done, 0));                           // the previous letterbox kernel must be done with d_raw
     for (int i = 0; i < n; ++i)
         B200_CHECK(cudaMemcpyAsync(e->d_raw + items[i].src_off, images[i], (size_t)widths[i] * heights[i] * 3 * esz, cudaMemcpyHostToDevice, up));
     B200_CHECK(cudaMemcpyAsync(e->d_lb_items, items.data(), (size_t)n * sizeof(LetterboxItem), cudaMemcpyHostToDevice, up));
     B200_CHECK(cudaMemcpyAsync(e->d_im_dims[e->dims_cur ^ 1], dims.data(), dims.size() * sizeof(int), cudaMemcpyHostToDevice, up));
-    if (!lb_sync) {
-        B200_CHECK(cudaEventRecord(e->lb_uploaded, up));
-        B200_CHECK(cudaStreamWaitEvent(e->stream, e->lb_uploaded, 0));
-    }
+    B200_CHECK(cudaEventRecord(e->lb_uploaded, up));
+    B200_CHECK(cudaStreamWaitEvent(e->stream, e->lb_uploaded, 0));
     launch_letterbox(e->d_raw, u8, e->d_lb_items, n, e->d_input, net->w, net->h, e->stream);
     B200_CHECK(cudaEventRecord(e->lb_done, e->stream));
     B200_CHECK(cudaStreamSynchronize(up));                  // items / dims live on this stack frame
@@ -1494,9 +1519,7 @@ extern "C" void b200_submit_batch(network *net, const float *input)
     need_device(e, "b200_submit_batch");
     if (e->submitted) { fprintf(stderr, "b200-darknet: b200_submit_batch called twice without b200_detect_submitted\n"); abort(); }
     if (input == B200_INPUT_RESIDENT) {          // the batch is whatever the input buffer holds now: its forward pass starts here
-        const int use_raw = (!e->head_sync && e->raw_decode_ok && !e->heads.empty()) ? 1 : 0;
-        adopt_letterbox_dims(e);
-        forward_layers(e, net, 0, net->n, use_raw != 0);
+        enqueue_forward(e, net, 0);
         e->submitted = 1; e->fwd_enqueued = 1;
         return;
     }
@@ -1507,18 +1530,30 @@ extern "C" void b200_submit_batch(network *net, const float *input)
     e->submitted = 1;
 }
 
-// the serving loops' step after the current batch's tail is enqueued: submit `next_input` (may be NULL) and enqueue its forward pass
+// the batch b200_submit_batch handed over becomes current: unless its forward pass is already enqueued, the spare buffer
+// its copy went to becomes the input and the compute stream waits for that copy.  Returns the first layer still to
+// enqueue: 0, or net->n
+static int make_submitted_current(b200_engine *e, const network *net, const char *what)
+{
+    if (!e->submitted) { fprintf(stderr, "b200-darknet: %s without a submitted batch\n", what); abort(); }
+    int first = net->n;
+    if (!e->fwd_enqueued) {
+        float *t = e->d_input; e->d_input = e->d_input_next; e->d_input_next = t;
+        B200_CHECK(cudaStreamWaitEvent(e->stream, e->submit_done, 0));
+        first = 0;
+    }
+    e->submitted = 0; e->fwd_enqueued = 0;
+    return first;
+}
+
+// the serving loops' step after the current batch's tail is enqueued: submit `next_input` (may be NULL) and enqueue its forward
+// pass, so that the next call finds that batch submitted with its forward pass in the stream
 static void enqueue_next_batch(b200_engine *e, network *net, const float *next_input)
 {
     if (!next_input) return;
     b200_submit_batch(net, next_input);
-    if (next_input == B200_INPUT_RESIDENT) return;                                   // forward enqueued by the submit
-    float *t = e->d_input; e->d_input = e->d_input_next; e->d_input_next = t;
-    B200_CHECK(cudaStreamWaitEvent(e->stream, e->submit_done, 0));
-    const int use_raw = (!e->head_sync && e->raw_decode_ok && !e->heads.empty()) ? 1 : 0;
-    adopt_letterbox_dims(e);
-    forward_layers(e, net, 0, net->n, use_raw != 0);
-    e->fwd_enqueued = 1;
+    enqueue_forward(e, net, make_submitted_current(e, net, "b200_submit_batch"));
+    e->submitted = 1; e->fwd_enqueued = 1;
 }
 
 extern "C" int b200_detect_submitted(network *net, const float *next_input, int w, int h, float thresh, float nms_thresh,
@@ -1527,14 +1562,7 @@ extern "C" int b200_detect_submitted(network *net, const float *next_input, int 
     b200_engine *e = b200_engine_of(net);
     need_device(e, "b200_detect_submitted");
     if (refuse_classifier(e, "b200_detect_submitted")) return -1;
-    if (!e->submitted) { fprintf(stderr, "b200-darknet: b200_detect_submitted without a submitted batch\n"); abort(); }
-    int first = net->n;                                                              // forward already enqueued by the previous call?
-    if (!e->fwd_enqueued) {
-        float *t = e->d_input; e->d_input = e->d_input_next; e->d_input_next = t;        // the submitted batch becomes current
-        B200_CHECK(cudaStreamWaitEvent(e->stream, e->submit_done, 0));
-        first = 0;
-    }
-    e->submitted = 0; e->fwd_enqueued = 0;
+    const int first = make_submitted_current(e, net, "b200_detect_submitted");
     // Once this batch's decode / NMS / collect are in the stream, the NEXT batch's copy is submitted and its whole forward pass
     // is enqueued behind them; the results of this batch are then read back on a separate stream while that forward runs.
     // (Waiting for the results first left the GPU idle for the two D2H round trips: ~0.25 ms of every 5 ms step.)
@@ -1574,8 +1602,7 @@ static int classify_core(b200_engine *e, network *net, int first, int top, int *
         e->d_top_cls = (int *)dev_alloc((size_t)e->cap * 64 * sizeof(int));
         e->d_top_prob = (float *)dev_alloc((size_t)e->cap * 64 * sizeof(float));
     }
-    if (first < net->n) adopt_letterbox_dims(e);
-    forward_layers(e, net, first, net->n);
+    enqueue_forward(e, net, first);
     launch_topk(e->L[e->cls_layer].head_out, batch, l.outputs, l.outputs, top, e->d_top_cls, e->d_top_prob, e->stream);
     B200_CHECK(cudaEventRecord(e->tail_done, e->stream));
     B200_CHECK(cudaStreamWaitEvent(e->d2h_stream, e->tail_done, 0));
@@ -1591,7 +1618,7 @@ extern "C" int b200_classify_batch(network *net, const float *input, int top, in
     b200_engine *e = b200_engine_of(net);
     need_device(e, "b200_classify_batch");
     if (!classify_args_ok(e, net, top, "b200_classify_batch")) return -1;
-    const int first = (input && input != B200_INPUT_RESIDENT) ? stage_input(e, net, input) : 0;
+    const int first = stage_batch_input(e, net, input);
     const int n = classify_core(e, net, first, top, classes, probs, [] {});
     B200_CHECK(cudaStreamSynchronize(e->stream));
     return n;
@@ -1602,14 +1629,7 @@ extern "C" int b200_classify_submitted(network *net, const float *next_input, in
     b200_engine *e = b200_engine_of(net);
     need_device(e, "b200_classify_submitted");
     if (!classify_args_ok(e, net, top, "b200_classify_submitted")) return -1;
-    if (!e->submitted) { fprintf(stderr, "b200-darknet: b200_classify_submitted without a submitted batch\n"); abort(); }
-    int first = net->n;
-    if (!e->fwd_enqueued) {
-        float *t = e->d_input; e->d_input = e->d_input_next; e->d_input_next = t;
-        B200_CHECK(cudaStreamWaitEvent(e->stream, e->submit_done, 0));
-        first = 0;
-    }
-    e->submitted = 0; e->fwd_enqueued = 0;
+    const int first = make_submitted_current(e, net, "b200_classify_submitted");
     return classify_core(e, net, first, top, classes, probs, [&] { enqueue_next_batch(e, net, next_input); });
 }
 
