@@ -87,16 +87,18 @@ void launch_local(TView in, TView out, const void *w, const float *bias, int siz
 }
 
 // ---- connected -------------------------------------------------------------------------------------------
-template <typename T, bool EXACT>
+// TI = input, TW = weights.  They differ after another [connected] (or [softmax]) in bf16 mode: those layers write fp32 rows.
+template <typename TI, typename TW, bool EXACT>
 __global__ void __launch_bounds__(256)
-connected_kernel(const T *__restrict__ in, int N, int K, int O, const T *__restrict__ wt, const float *__restrict__ scale,
+connected_kernel(const TI *__restrict__ in, int N, int K, int O, const TW *__restrict__ wt, const float *__restrict__ scale,
                  const float *__restrict__ shift, int act, float *__restrict__ out)
 {
-    constexpr int V = Elem<T>::VEC;
+    constexpr int V = Elem<TW>::VEC, VI = Elem<TI>::VEC;
+    static_assert(V % VI == 0, "one weight vector spans whole input vectors");
     const int lane = threadIdx.x & 31;
     const int o = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (o >= O) return;
-    const T *wrow = wt + (size_t)o * K;
+    const TW *wrow = wt + (size_t)o * K;
     const int Kv = K - K % V;
     for (int b0 = 0; b0 < N; b0 += DENSE_BT) {
         float acc[DENSE_BT];
@@ -104,16 +106,18 @@ connected_kernel(const T *__restrict__ in, int N, int K, int O, const T *__restr
         for (int i = 0; i < DENSE_BT; ++i) acc[i] = 0.f;
         for (int k = lane * V; k < Kv; k += 32 * V) {
             float wv[V];
-            load_vec<T>(wrow + k, wv);
+            load_vec<TW>(wrow + k, wv);
 #pragma unroll
             for (int i = 0; i < DENSE_BT; ++i)
-                if (b0 + i < N) fma_vec<T>(wv, in + (size_t)(b0 + i) * K + k, acc[i]);
+                if (b0 + i < N)
+#pragma unroll
+                    for (int j = 0; j < V; j += VI) fma_vec<TI>(wv + j, in + (size_t)(b0 + i) * K + k + j, acc[i]);
         }
         for (int k = Kv + lane; k < K; k += 32) {               // scalar tail when K is not a multiple of the vector width
-            float wv = Elem<T>::load(wrow + k);
+            float wv = Elem<TW>::load(wrow + k);
 #pragma unroll
             for (int i = 0; i < DENSE_BT; ++i)
-                if (b0 + i < N) acc[i] = fmaf(wv, Elem<T>::load(in + (size_t)(b0 + i) * K + k), acc[i]);
+                if (b0 + i < N) acc[i] = fmaf(wv, Elem<TI>::load(in + (size_t)(b0 + i) * K + k), acc[i]);
         }
 #pragma unroll
         for (int i = 0; i < DENSE_BT; ++i) {
@@ -126,14 +130,16 @@ connected_kernel(const T *__restrict__ in, int N, int K, int O, const T *__restr
 void launch_connected(const void *in, int in_dtype, int batch, int inputs, int outputs, const void *w, int w_dtype,
                       const float *scale, const float *shift, int act, float *out, cudaStream_t s)
 {
-    if (in_dtype != w_dtype) { fprintf(stderr, "b200-darknet: connected layer dtype mismatch\n"); abort(); }
     int grid = div_up((long long)outputs * 32, 256);
     bool aligned = ((uintptr_t)in % 16 == 0) && ((uintptr_t)w % 16 == 0) && (inputs % Elem<bf16>::VEC == 0);
     if (!aligned) { fprintf(stderr, "b200-darknet: connected layer needs 16-byte aligned rows (inputs %% 8 == 0)\n"); abort(); }
-    if (in_dtype == DT_F32)
-        connected_kernel<float, true><<<grid, 256, 0, s>>>((const float *)in, batch, inputs, outputs, (const float *)w, scale, shift, act, out);
-    else
-        connected_kernel<bf16, false><<<grid, 256, 0, s>>>((const bf16 *)in, batch, inputs, outputs, (const bf16 *)w, scale, shift, act, out);
+    if (in_dtype == DT_F32 && w_dtype == DT_F32)
+        connected_kernel<float, float, true><<<grid, 256, 0, s>>>((const float *)in, batch, inputs, outputs, (const float *)w, scale, shift, act, out);
+    else if (in_dtype == DT_BF16 && w_dtype == DT_BF16)
+        connected_kernel<bf16, bf16, false><<<grid, 256, 0, s>>>((const bf16 *)in, batch, inputs, outputs, (const bf16 *)w, scale, shift, act, out);
+    else if (in_dtype == DT_F32 && w_dtype == DT_BF16)
+        connected_kernel<float, bf16, false><<<grid, 256, 0, s>>>((const float *)in, batch, inputs, outputs, (const bf16 *)w, scale, shift, act, out);
+    else { fprintf(stderr, "b200-darknet: connected layer: unsupported input / weight dtype pair\n"); abort(); }
     B200_LAUNCHED();
 }
 

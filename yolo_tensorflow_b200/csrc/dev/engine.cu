@@ -12,6 +12,7 @@
 #include "engine.h"
 #include <cmath>
 #include <cstring>
+#include <functional>
 
 static void *dev_alloc(size_t bytes)
 {
@@ -249,6 +250,16 @@ static void plan_outputs(b200_engine *e, const network *net, const std::vector<s
         e->L[i].cls_logits = net->layers[i].type == CONVOLUTIONAL &&
                              (only_consumer_is(i, SOFTMAX) || (only_consumer_is(i, AVGPOOL) && only_consumer_is(i + 1, SOFTMAX)));
 
+    // does a [connected] read layer j's buffer, directly or through the aliases [dropout] and a one-input [route]?  It reads
+    // dense rows (launch_connected, connected_tc), so such a convolution keeps its row pitch at its filter count
+    std::function<bool(int)> read_by_connected = [&](int j) {
+        for (int c : cons[j]) {
+            const layer &cl = net->layers[c];
+            if (cl.type == CONNECTED || ((cl.type == DROPOUT || (cl.type == ROUTE && cl.n == 1)) && read_by_connected(c))) return true;
+        }
+        return false;
+    };
+
     // output views
     size_t max_floats = (size_t)e->cap * net->inputs;
     for (int i = 0; i < net->n; ++i) {
@@ -266,8 +277,9 @@ static void plan_outputs(b200_engine *e, const network *net, const std::vector<s
         switch (l.type) {
         case CONVOLUTIONAL: {
             // row pitch padded to 16 filters (255 -> 256): keeps every pixel row 16-byte aligned for vector stores; a classifier's
-            // logits to 64 (1000 -> 1024), whole 64-filter tiles of the tcgen05 GEMM like the connected layer's
-            int ld = (int)align_up(l.out_c, d.cls_logits ? 64 : 16);
+            // logits to 64 (1000 -> 1024), whole 64-filter tiles of the tcgen05 GEMM like the connected layer's; dense when a
+            // [connected] reads it (conv_tc_plan_create refuses a pitch below the padded filter count: conv_simt runs then)
+            int ld = read_by_connected(i) ? l.out_c : (int)align_up(l.out_c, d.cls_logits ? 64 : 16);
             if (d.fused_into >= 0) {            // written straight into the shortcut's buffer, never materialised
                 d.out = TView{nullptr, e->cap, l.out_h, l.out_w, l.out_c, ld, dtype};
                 d.owns_out = false;
@@ -373,6 +385,8 @@ static void plan_arena(b200_engine *e, const network *net)
 // every layer's kernel and tcgen05 plan; a fusion whose shapes the plan does not take is undone here
 static void select_kernels(b200_engine *e, const network *net, const std::vector<std::vector<int>> &cons, const std::vector<int> &place_route)
 {
+    // what layer i reads: the previous layer's output, or for the first layer the converted image (run_layer's `in`)
+    auto input_of = [&](int i) { return i > 0 ? e->L[i - 1].out : e->in_view; };
     for (int i = 0; i < net->n; ++i) {
         const layer &l = net->layers[i];
         DevLayer &d = e->L[i];
@@ -400,16 +414,16 @@ static void select_kernels(b200_engine *e, const network *net, const std::vector
                 }
                 if (d.fused_into >= 0) {
                     const layer &sc = net->layers[d.fused_into];
-                    d.tc = conv_tc_plan_create(e->L[i - 1].out, e->L[d.fused_into].out, p, &e->L[sc.index].out, sc.alpha, sc.beta);
+                    d.tc = conv_tc_plan_create(input_of(i), e->L[d.fused_into].out, p, &e->L[sc.index].out, sc.alpha, sc.beta);
                     if (!d.tc) { fprintf(stderr, "b200-darknet: internal error: fused conv %d has no tcgen05 plan\n", i); abort(); }
                     d.kernel = "conv_tc+shortcut";
                 } else {
                     if (d.up_fused) {
-                        d.tc = conv_tc_plan_create(e->L[i - 1].out, d.out, p, nullptr, 1.f, 1.f, &e->L[i + 1].out);
+                        d.tc = conv_tc_plan_create(input_of(i), d.out, p, nullptr, 1.f, 1.f, &e->L[i + 1].out);
                         if (d.tc) { d.kernel = "conv_tc+upsample"; break; }
                         d.up_fused = false; e->L[i + 1].up_away = false;           // shape not covered: the two layers run separately
                     }
-                    d.tc = conv_tc_plan_create(e->L[i - 1].out, d.out, p, nullptr, 1.f, 1.f);
+                    d.tc = conv_tc_plan_create(input_of(i), d.out, p, nullptr, 1.f, 1.f);
                     if (d.tc) d.kernel = "conv_tc";
                 }
             }
@@ -455,7 +469,7 @@ static void select_kernels(b200_engine *e, const network *net, const std::vector
                 // 49 independent GEMMs [images x 9C] x [9C x filters]: the conv kernel with one pixel per tile and the weight
                 // box taken from that pixel's own slab
                 ConvParams p{l.size, l.stride, l.pad, act_id(l.activation), d.w, d.scale, d.lbias, l.n};
-                d.tc = conv_tc_plan_create(e->L[i - 1].out, d.out, p, nullptr, 1.f, 1.f, nullptr, 1);
+                d.tc = conv_tc_plan_create(input_of(i), d.out, p, nullptr, 1.f, 1.f, nullptr, 1);
                 if (d.tc) d.kernel = "local_tc";
             }
             break;
